@@ -20,9 +20,13 @@ One "step" = one epoch of the hot path: T=1000 fused forward/sample/store launch
 
 Both arms run on ONE set of trainer objects (policy, optimizer state, buffer): the `value`
 arm's W warm-up epochs warm every kernel of the `e2e` arm as well, which only swaps the rollout
-front end (one extra warm-up epoch covers its copy path).  A wall-clock budget
-(SPO_BENCH_BUDGET_S, default 780 s -- the driver's per-run limit is 870 s) bounds the e2e
-arm: if K more epochs would not fit, it times fewer and says so in `e2e.steps`.
+front end (one extra warm-up epoch covers its copy path).  Each arm times exactly K epochs.
+
+--dump-outputs DIR writes, after the timed epochs of the `value` arm, what its last epoch
+handed back as DIR/<name>.npy (rank 0): the trained policy's parameters under their
+state_dict names, the update's statistics, the Lagrange multiplier and a fixed, seeded
+sample of rows of the epoch's batch.  The inputs depend on the arguments only, so two
+builds run with the same arguments can be compared output for output.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md section "Measurement" for the roofline and
 cpu_baseline definitions.
@@ -77,10 +81,6 @@ def bytes_per_sample_update():
     return 4 * (D_OBS + D_ACT + 4) + 8
 
 
-T_START = time.time()
-BUDGET_S = float(os.environ.get("SPO_BENCH_BUDGET_S", "780"))
-
-
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -96,7 +96,12 @@ def parse():
                     help="steps per env of the reference arm's measured mini-epoch (0 = sized from --cpu-seconds)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed epoch computed as DIR/<name>.npy (e.g. bench_outputs/)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -251,7 +256,31 @@ def timed_epochs(tr, K, W, world, device):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     return dict(ms=ms, launches=L.LAUNCHES["n"] - l0, stops=stops, msteps=msteps, clocks=clk.summary(),
-                h2d=(tr["roll"].bytes_h2d - h0) / K, d2h=(tr["roll"].bytes_d2h - d0) / K)
+                h2d=(tr["roll"].bytes_h2d - h0) / K, d2h=(tr["roll"].bytes_d2h - d0) / K, last=res)
+
+
+DUMP_ROWS = 65536   # batch rows dumped: 65536 x 4 (D + A + 11) bytes, 26 MB at the largest workload (cpo, D = 88)
+
+
+def dump_outputs(tr, last, out_dir):
+    """Write what the epoch just run handed back: the policy's parameters, the update's statistics, the Lagrange
+    multiplier and the rows of a fixed, seeded sample of the epoch's batch (every field buffer.get() returned)."""
+    S = tr["N"] * tr["T"]
+    rows = np.sort(np.random.default_rng(0).choice(S, min(S, DUMP_ROWS), replace=False))
+    idx = torch.as_tensor(rows, device=tr["device"])
+    out = {f"policy.{k}": v for k, v in tr["policy"].state_dict().items()}
+    for k, v in tr["buffer"].data.items():
+        out[f"batch.{k}"] = v.reshape(S, *v.shape[2:])[idx]
+    out["batch.adv"] = tr["buffer"].adv_mixed[idx]
+    out["batch.row_index"] = rows.astype(np.float64)
+    for k, v in last.items():
+        out[f"update.{k}"] = np.float64(v)
+    if tr["lagrange"] is not None:
+        out["lagrange.multiplier"] = np.float64(tr["lagrange"].lagrangian_multiplier)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def time_dominant_kernel(tr, device):
@@ -410,6 +439,8 @@ def run_spo(args):
         dp = DataParallel()
     tr = build_trainer(args, device, rank, resident=True, dp=dp)
     val = timed_epochs(tr, K, W, world, device)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(tr, val["last"], args.dump_outputs)      # before time_dominant_kernel trains the policy further
     dom = time_dominant_kernel(tr, device) if world == 1 else None
     e2e = None
     if not args.no_e2e:
@@ -420,16 +451,7 @@ def run_spo(args):
         env2 = SyntheticVecEnv(args.num_envs, D_OBS, D_ACT, episode_len=args.horizon, seed=rank)
         tr2["env"] = env2
         tr2["roll"] = Rollout(env2, tr["policy"], tr["buffer"], tr["logger"], tr["roll"].args, device)
-        epoch_s = val["ms"] / K / 1e3 * 1.10 + 0.5
-        reserve = 0.0 if (args.no_cpu_baseline or world > 1) else args.cpu_seconds + 10.0
-        left = BUDGET_S - (time.time() - T_START) - reserve
-        k_e = int(min(K, max(1, int(left / epoch_s) - 1)))      # -1: the warm-up epoch
-        if world > 1:
-            t = torch.tensor([k_e], device=device)
-            dist.broadcast(t, src=0)
-            k_e = int(t.item())
-        e2e = timed_epochs(tr2, k_e, 1, world, device)
-        e2e["K"] = k_e
+        e2e = timed_epochs(tr2, K, 1, world, device)
     if dp is not None:
         dp.close()
 
@@ -481,8 +503,8 @@ def run_spo(args):
     if "critic_pass_ms" in dom:
         out["config"]["ms_per_critic_regression_pass"] = dom["critic_pass_ms"]
     if e2e is not None:
-        out["e2e"] = {"value": S * e2e["K"] * world / (e2e["ms"] / 1e3), "unit": "env-steps/s", "h2d_bytes_per_step": e2e["h2d"],
-                      "d2h_bytes_per_step": e2e["d2h"], "ms_per_step": e2e["ms"] / e2e["K"], "steps": e2e["K"], "warmup": 1,
+        out["e2e"] = {"value": S * K * world / (e2e["ms"] / 1e3), "unit": "env-steps/s", "h2d_bytes_per_step": e2e["h2d"],
+                      "d2h_bytes_per_step": e2e["d2h"], "ms_per_step": e2e["ms"] / K, "steps": K, "warmup": 1,
                       "stop_iter": e2e["stops"], "gpu_launches": e2e["launches"],
                       "note": "same trainer objects as the value arm (already warm); only the rollout front end differs"}
     if not args.no_cpu_baseline:

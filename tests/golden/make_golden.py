@@ -217,6 +217,10 @@ def gen_update_chain(ref, out):
                 kls.append(torch.distributions.kl.kl_divergence(od, nd).sum(-1, keepdim=True).mean().item())
         res[kind] = dict(D=D, A=A, init=init, data=data, lam=lam, perms=perms, losses=torch.tensor(losses),
                          kls=torch.tensor(kls), final=state_of(pol), batch=B)
+    # both kinds start from the same seeded weights, data and minibatch orders: the file keeps one copy of them
+    for key in ("init", "data", "perms"):
+        torch.testing.assert_close(res["focops"][key], res["ppo"][key], rtol=0, atol=0)
+        res["focops"][key] = res["ppo"][key]
     out["update_chain"] = res
 
 
