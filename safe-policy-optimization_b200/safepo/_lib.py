@@ -59,6 +59,66 @@ CTRL_KL_SUM_F64_INDEX = 3        # byte offset 24
 
 LOSS_PPO_CLIP, LOSS_FOCOPS, LOSS_CRITIC_ONLY, LOSS_PG, LOSS_CUP_PROJECTION = 0, 1, 2, 3, 4
 
+_i, _i64, _f, _d, _u64, _p = C.c_int, C.c_int64, C.c_float, C.c_double, C.c_uint64, C.c_void_p
+_pi, _PD = C.POINTER(C.c_int), C.POINTER(Dims)
+
+# Every entry point of include/spo.h: name -> (argtypes, whether a call counts as a kernel launch in LAUNCHES).
+# spo_conjugate_gradient launches 2 * iters + 1 kernels; its caller counts them.
+_ABI = {
+    "spo_version": ([], False),
+    "spo_last_error": ([], False),
+    "spo_sync_check": ([_p], False),
+    "spo_param_count": ([_PD, _pi, _pi, _pi], False),
+    "spo_param_offsets": ([_PD, _i] + [_pi] * 7, False),
+    "spo_policy_step": ([_PD, _p, _p, _p, _u64, _u64, _i, _i, _p, _p, _p, _p, C.POINTER(Rollout), _i, _p], True),
+    "spo_critic_values": ([_PD, _p, _p, _i, _p, _p, _p], True),
+    "spo_store_transition": ([C.POINTER(Rollout), _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p], True),
+    "spo_gae_dual": ([_p, _p, _p, _p, _p, _p, _p, _f, _d, _d, _p, _p, _p, _p, _i, _i, _i, _p], True),
+    "spo_adv_stats": ([_p, _p, _i64, _p, _p], True),
+    "spo_adv_apply": ([_p, _p, _i64, _p, _i, _i, _f, _f, _p, _p], True),
+    "spo_pg_update": ([_PD, _p, _p, _p, _p, C.POINTER(Batch), _p, _i64, _i, _i, C.POINTER(HParams), _p, _p], True),
+    "spo_comm_slot_floats": ([_PD, _pi], False),
+    "spo_pg_update_dp": ([_PD, _p, _p, _p, _p, C.POINTER(Batch), _p, _i64, _i, _i, C.POINTER(HParams), _p, C.POINTER(Comm), _p],
+                         True),
+    "spo_comm_alloc": ([C.c_size_t, C.POINTER(_p)], False),
+    "spo_comm_free": ([_p], False),
+    "spo_comm_export": ([_p, C.c_char_p], False),
+    "spo_comm_import": ([C.c_char_p, C.POINTER(_p)], False),
+    "spo_comm_close": ([_p], False),
+    "spo_actor_kl_accumulate": ([_PD, _p, _p, _p, _p, _i64, _p, _p], True),
+    "spo_kl_finalize": ([_p, _d, _f, _p], True),
+    "spo_actor_forward": ([_PD, _p, _p, _i64, _p, _p], True),
+    "spo_actor_kl": ([_PD, _p, _p, _p, _p, _i64, _i, _f, _p, _p], True),
+    "spo_surrogate_grad": ([_PD, _p, _p, _p, _p, _p, _i64, _p, _p, _p], True),
+    "spo_fvp": ([_PD, _p, _p, _i64, _p, _f, _p, _p], True),
+    "spo_linesearch_eval": ([_PD, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p], True),
+    "spo_conjugate_gradient": ([_PD, _p, _p, _i64, _p, _i, _f, _f, _f, _p, _p, _p], False),
+    "spo_cg_begin": ([_PD, _p, _p, _p, _p], True),
+    "spo_cg_update": ([_PD, _p, _p, _f, _f, _p], True),
+    "spo_obs_normalize": ([_p, _i, _i, _p, _p, _d, _p, _i, _d, _p, _p], True),
+    "spo_action_rescale": ([_p, _i, _i, _p, _p, _f, _f, _p, _p], True),
+    "spo_gae_masked": ([_p, _p, _p, _f, _f, _f, _d, _p, _i, _i, _p], True),
+    "spo_ma_mlp_layer": ([_p, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p], True),
+    "spo_ma_head": ([_p, _i, _i, _p, _p, _i, _p, _f, _f, _p, _p, _p, _p], True),
+    "spo_ma_mlp_layer_train": ([_p, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p], True),
+    "spo_ma_ln_elu_bwd": ([_p, _p, _p, _i, _i, _p, _p, _p], True),
+    "spo_ma_ln_in_bwd": ([_p, _p, _i, _i, _p, _p], True),
+    "spo_ma_partial_reduce": ([_p, _i, _i, _i, _i, _p, _p, _p, _f, _p], True),
+    "spo_ma_gemm_nn": ([_p, _p, _p, _i, _i, _i, _p], True),
+    "spo_ma_gemm_tn": ([_p, _p, _p, _i, _i, _i, _i, _p], True),
+    "spo_ma_actor_loss": ([_p, _i, _i, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _f, _f, _f, _f, _p, _p, _p, _p], True),
+    "spo_ma_actor_finalize": ([_p, _i, _i, _p, _i, _f, _f, _f, _p, _p, _p, _p], True),
+    "spo_ma_value_loss": ([_p, _p, _p, _p, _i, _f, _f, _f, _p, _p, _p], True),
+    "spo_ma_popart_normalize": ([_p, _i, _p, _d, _f, _p, _p], True),
+    "spo_ma_lagrange_step": ([_p, _p, _p, _i, _f, _d, _f, _p, _p], True),
+    "spo_ma_clip_adam": ([_p, _p, _p, _p, _i, _f, _d, _d, _d, _d, _d, _i, _p, _p, _p], True),
+}
+EXPORTS = tuple(_ABI)
+_KERNEL_CALLS = frozenset(name for name, (_, launch) in _ABI.items() if launch)
+
+# number of libspo kernels launched so far (bench.py reports the delta over its timed region)
+LAUNCHES = {"n": 0}
+
 _lib = None
 
 
@@ -69,83 +129,12 @@ def lib():
             raise SpoError(f"{LIB_PATH} not found: build it with `python safe-policy-optimization_b200/build.py` "
                            "(there is no CPU / PyTorch fallback for the hot path)")
         _lib = C.CDLL(LIB_PATH)
+        for name, (argtypes, _) in _ABI.items():
+            fn = getattr(_lib, name)
+            fn.argtypes = argtypes
+            fn.restype = C.c_int
         _lib.spo_last_error.restype = C.c_char_p
-        _declare(_lib)
     return _lib
-
-
-def _declare(L):
-    i, i64, f, d, u64, p = C.c_int, C.c_int64, C.c_float, C.c_double, C.c_uint64, C.c_void_p
-    PD = C.POINTER(Dims)
-    sig = {
-        "spo_version": [],
-        "spo_sync_check": [p],
-        "spo_param_count": [PD, C.POINTER(i), C.POINTER(i), C.POINTER(i)],
-        "spo_param_offsets": [PD, i] + [C.POINTER(i)] * 7,
-        "spo_policy_step": [PD, p, p, p, u64, u64, i, i, p, p, p, p, C.POINTER(Rollout), i, p],
-        "spo_critic_values": [PD, p, p, i, p, p, p],
-        "spo_store_transition": [C.POINTER(Rollout), i, p, p, p, p, i, p, p, p, p, p],
-        "spo_gae_dual": [p, p, p, p, p, p, p, f, d, d, p, p, p, p, i, i, i, p],
-        "spo_adv_stats": [p, p, i64, p, p],
-        "spo_adv_apply": [p, p, i64, p, i, i, f, f, p, p],
-        "spo_pg_update": [PD, p, p, p, p, C.POINTER(Batch), p, i64, i, i, C.POINTER(HParams), p, p],
-        "spo_comm_slot_floats": [PD, C.POINTER(i)],
-        "spo_pg_update_dp": [PD, p, p, p, p, C.POINTER(Batch), p, i64, i, i, C.POINTER(HParams), p, C.POINTER(Comm), p],
-        "spo_comm_alloc": [C.c_size_t, C.POINTER(p)],
-        "spo_comm_free": [p],
-        "spo_comm_export": [p, C.c_char_p],
-        "spo_comm_import": [C.c_char_p, C.POINTER(p)],
-        "spo_comm_close": [p],
-        "spo_actor_kl_accumulate": [PD, p, p, p, p, i64, p, p],
-        "spo_kl_finalize": [p, d, f, p],
-        "spo_actor_forward": [PD, p, p, i64, p, p],
-        "spo_actor_kl": [PD, p, p, p, p, i64, i, f, p, p],
-        "spo_surrogate_grad": [PD, p, p, p, p, p, i64, p, p, p],
-        "spo_fvp": [PD, p, p, i64, p, f, p, p],
-        "spo_linesearch_eval": [PD, p, p, p, p, p, p, p, p, i64, p, p],
-        "spo_conjugate_gradient": [PD, p, p, i64, p, i, f, f, f, p, p, p],
-        "spo_ma_mlp_layer": [p, i, i, p, p, p, p, i, p, p, p, p],
-        "spo_ma_head": [p, i, i, p, p, i, p, f, f, p, p, p, p],
-        "spo_ma_mlp_layer_train": [p, i, i, p, p, p, p, i, p, p, p, p, p, p],
-        "spo_ma_ln_elu_bwd": [p, p, p, i, i, p, p, p],
-        "spo_ma_ln_in_bwd": [p, p, i, i, p, p],
-        "spo_ma_partial_reduce": [p, i, i, i, i, p, p, p, f, p],
-        "spo_ma_gemm_nn": [p, p, p, i, i, i, p],
-        "spo_ma_gemm_tn": [p, p, p, i, i, i, i, p],
-        "spo_ma_actor_loss": [p, i, i, p, p, p, i, p, p, p, p, p, p, f, f, f, f, p, p, p, p],
-        "spo_ma_actor_finalize": [p, i, i, p, i, f, f, f, p, p, p, p],
-        "spo_ma_value_loss": [p, p, p, p, i, f, f, f, p, p, p],
-        "spo_ma_popart_normalize": [p, i, p, d, f, p, p],
-        "spo_ma_lagrange_step": [p, p, p, i, f, d, f, p, p],
-        "spo_ma_clip_adam": [p, p, p, p, i, f, d, d, d, d, d, i, p, p, p],
-        "spo_cg_begin": [PD, p, p, p, p],
-        "spo_cg_update": [PD, p, p, f, f, p],
-        "spo_obs_normalize": [p, i, i, p, p, d, p, i, d, p, p],
-        "spo_action_rescale": [p, i, i, p, p, f, f, p, p],
-        "spo_gae_masked": [p, p, p, f, f, f, d, p, i, i, p],
-    }
-    for name, args in sig.items():
-        fn = getattr(L, name)
-        fn.argtypes = args
-        fn.restype = C.c_int
-
-
-EXPORTS = ("spo_version", "spo_last_error", "spo_sync_check", "spo_param_count", "spo_param_offsets",
-           "spo_policy_step", "spo_critic_values", "spo_store_transition", "spo_gae_dual", "spo_adv_stats",
-           "spo_adv_apply", "spo_pg_update", "spo_actor_forward", "spo_actor_kl", "spo_surrogate_grad", "spo_fvp",
-           "spo_linesearch_eval", "spo_conjugate_gradient", "spo_comm_slot_floats", "spo_pg_update_dp", "spo_comm_alloc",
-           "spo_comm_free", "spo_comm_export", "spo_comm_import", "spo_comm_close", "spo_actor_kl_accumulate", "spo_kl_finalize",
-           "spo_obs_normalize", "spo_action_rescale", "spo_gae_masked", "spo_cg_begin", "spo_cg_update", "spo_ma_mlp_layer", "spo_ma_head",
-           "spo_ma_mlp_layer_train", "spo_ma_ln_elu_bwd", "spo_ma_ln_in_bwd", "spo_ma_partial_reduce", "spo_ma_gemm_nn", "spo_ma_gemm_tn", "spo_ma_actor_loss", "spo_ma_actor_finalize", "spo_ma_value_loss", "spo_ma_popart_normalize", "spo_ma_lagrange_step", "spo_ma_clip_adam")
-
-
-# number of libspo kernels launched so far (bench.py reports the delta over its timed region)
-LAUNCHES = {"n": 0}
-_KERNEL_CALLS = {"spo_policy_step", "spo_critic_values", "spo_store_transition", "spo_gae_dual", "spo_adv_stats",
-                 "spo_adv_apply", "spo_pg_update", "spo_actor_forward", "spo_actor_kl", "spo_surrogate_grad", "spo_fvp",
-                 "spo_linesearch_eval", "spo_pg_update_dp", "spo_actor_kl_accumulate", "spo_kl_finalize", "spo_obs_normalize",
-                 "spo_action_rescale", "spo_gae_masked", "spo_cg_begin", "spo_cg_update", "spo_ma_mlp_layer", "spo_ma_head",
-                 "spo_ma_mlp_layer_train", "spo_ma_ln_elu_bwd", "spo_ma_ln_in_bwd", "spo_ma_partial_reduce", "spo_ma_gemm_nn", "spo_ma_gemm_tn", "spo_ma_actor_loss", "spo_ma_actor_finalize", "spo_ma_value_loss", "spo_ma_popart_normalize", "spo_ma_lagrange_step", "spo_ma_clip_adam"}
 
 
 def check(rc, what):
@@ -153,6 +142,11 @@ def check(rc, what):
         LAUNCHES["n"] += 1
     if rc != 0:
         raise SpoError(f"{what} failed ({rc}): {lib().spo_last_error().decode()}")
+
+
+def call(name, *args):
+    """Call entry point ``name`` of the library, count it in LAUNCHES if it is a kernel, raise SpoError on failure."""
+    check(getattr(lib(), name)(*args), name)
 
 
 def ptr(t):
@@ -176,11 +170,11 @@ def dims(obs_dim, act_dim, hidden=64):
 
 def param_count(d):
     a, c, t = C.c_int(), C.c_int(), C.c_int()
-    check(lib().spo_param_count(C.byref(d), C.byref(a), C.byref(c), C.byref(t)), "spo_param_count")
+    call("spo_param_count", C.byref(d), C.byref(a), C.byref(c), C.byref(t))
     return a.value, c.value, t.value
 
 
 def param_offsets(d, net):
     out = [C.c_int() for _ in range(7)]
-    check(lib().spo_param_offsets(C.byref(d), net, *[C.byref(o) for o in out]), "spo_param_offsets")
+    call("spo_param_offsets", C.byref(d), net, *[C.byref(o) for o in out])
     return dict(zip(("log_std", "w1", "b1", "w2", "b2", "w3", "b3"), (o.value for o in out)))

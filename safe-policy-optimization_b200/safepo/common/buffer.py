@@ -86,33 +86,31 @@ class VectorizedOnPolicyBuffer:
         cost [N] float32; terminated, truncated [N] uint8; next_v / final_v = (v_r, v_c)."""
         nr, nc = next_v if next_v is not None else (None, None)
         fr, fc = final_v if final_v is not None else (None, None)
-        L.check(L.lib().spo_store_transition(C.byref(self.struct), int(t), L.ptr(reward), L.ptr(cost), L.ptr(terminated),
-                                             L.ptr(truncated), int(bool(epoch_end)), L.ptr(nr), L.ptr(nc), L.ptr(fr),
-                                             L.ptr(fc), L.stream()), "spo_store_transition")
+        L.call("spo_store_transition", C.byref(self.struct), int(t), L.ptr(reward), L.ptr(cost), L.ptr(terminated),
+               L.ptr(truncated), int(bool(epoch_end)), L.ptr(nr), L.ptr(nc), L.ptr(fr),
+               L.ptr(fc), L.stream())
         self.ptr_list = [int(t) + 1] * self.num_envs
 
     def compute_gae(self):
         d = self.data
-        L.check(L.lib().spo_gae_dual(L.ptr(d["reward"]), L.ptr(d["cost"]), L.ptr(d["value_r"]), L.ptr(d["value_c"]),
-                                     L.ptr(self.seg_end), L.ptr(self.boot_r), L.ptr(self.boot_c),
-                                     float(self._gamma), float(self._gamma * self._lam), float(self._gamma * self._lam_c),
-                                     L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), L.ptr(d["target_value_r"]),
-                                     L.ptr(d["target_value_c"]), self.num_envs, self.size, self.gae_mode, L.stream()),
-                "spo_gae_dual")
+        L.call("spo_gae_dual", L.ptr(d["reward"]), L.ptr(d["cost"]), L.ptr(d["value_r"]), L.ptr(d["value_c"]),
+               L.ptr(self.seg_end), L.ptr(self.boot_r), L.ptr(self.boot_c),
+               float(self._gamma), float(self._gamma * self._lam), float(self._gamma * self._lam_c),
+               L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), L.ptr(d["target_value_r"]),
+               L.ptr(d["target_value_c"]), self.num_envs, self.size, self.gae_mode, L.stream())
 
     def finalize(self, lagrangian_multiplier=0.0, all_reduce=None):
         """Statistics + standardisation (buffer.py:154-160) + Lagrange mix (ppo_lag.py:280-281).
         ``all_reduce(stats)``: optional hook summing the 4 fp64 statistics across ranks."""
         d = self.data
         S = self.num_envs * self.size
-        lib = L.lib()
-        L.check(lib.spo_adv_stats(L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), S, L.ptr(self.stats), L.stream()), "spo_adv_stats")
+        L.call("spo_adv_stats", L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), S, L.ptr(self.stats), L.stream())
         if all_reduce is not None:
             all_reduce(self.stats)
         lam = float(lagrangian_multiplier)
-        L.check(lib.spo_adv_apply(L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), S, L.ptr(self.stats),
-                                  int(self._standardized_adv_r), int(self._standardized_adv_c), lam, lam + 1,
-                                  L.ptr(self.adv_mixed), L.stream()), "spo_adv_apply")
+        L.call("spo_adv_apply", L.ptr(d["adv_r"]), L.ptr(d["adv_c"]), S, L.ptr(self.stats),
+               int(self._standardized_adv_r), int(self._standardized_adv_c), lam, lam + 1,
+               L.ptr(self.adv_mixed), L.stream())
         return self.adv_mixed
 
     def get(self, lagrangian_multiplier=0.0, all_reduce=None):
@@ -145,8 +143,8 @@ def masked_gae_returns(rewards, value_preds, masks, popart_mean, popart_sqrt_var
         raise L.SpoError("value_preds / masks must have T+1 time steps")
     if out is None:
         out = torch.empty_like(rewards)
-    L.check(L.lib().spo_gae_masked(L.ptr(rewards), L.ptr(value_preds), L.ptr(masks), float(popart_mean), float(popart_sqrt_var),
-                                   float(gamma), float(gamma) * float(gae_lambda), L.ptr(out), N, T, L.stream()), "spo_gae_masked")
+    L.call("spo_gae_masked", L.ptr(rewards), L.ptr(value_preds), L.ptr(masks), float(popart_mean), float(popart_sqrt_var),
+           float(gamma), float(gamma) * float(gae_lambda), L.ptr(out), N, T, L.stream())
     return out
 
 

@@ -69,19 +69,18 @@ class DataParallel:
 
     # ---- peer-mapped staging for the in-kernel gradient sum --------------------------------
     def setup_peer_buffers(self, dims, device):
-        lib = L.lib()
         slot = C.c_int()
-        L.check(lib.spo_comm_slot_floats(C.byref(dims), C.byref(slot)), "spo_comm_slot_floats")
+        L.call("spo_comm_slot_floats", C.byref(dims), C.byref(slot))
         nbytes_grad = 2 * self.world * 3 * slot.value * 4      # [parity][source rank][net][slot] 8-byte {value, sequence} words
         own = []
         for nbytes in (nbytes_grad, max(256, 4 * 3 * self.world)):
             ptr = C.c_void_p()
-            L.check(lib.spo_comm_alloc(nbytes, C.byref(ptr)), "spo_comm_alloc")
+            L.call("spo_comm_alloc", nbytes, C.byref(ptr))
             own.append(ptr.value)
         handles = []
         for ptr in own:
             buf = C.create_string_buffer(64)
-            L.check(lib.spo_comm_export(ptr, buf), "spo_comm_export")
+            L.call("spo_comm_export", ptr, buf)
             handles.append(buf.raw)
         gathered = [None] * self.world
         dist.all_gather_object(gathered, handles, group=self.group)
@@ -91,8 +90,8 @@ class DataParallel:
                 grads.append(own[0]); flags.append(own[1])
                 continue
             pg, pf = C.c_void_p(), C.c_void_p()
-            L.check(lib.spo_comm_import(hg, C.byref(pg)), "spo_comm_import")
-            L.check(lib.spo_comm_import(hf, C.byref(pf)), "spo_comm_import")
+            L.call("spo_comm_import", hg, C.byref(pg))
+            L.call("spo_comm_import", hf, C.byref(pf))
             grads.append(pg.value); flags.append(pf.value)
         self._peer = {
             "own": own, "grads": grads, "flags": flags,

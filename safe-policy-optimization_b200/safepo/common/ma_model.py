@@ -17,10 +17,6 @@ import torch
 from safepo import _lib as L
 
 
-def _launch(name, *args):
-    L.check(getattr(L.lib(), name)(*args), name)
-
-
 class _Net:
     def __init__(self, state, device, layer_N):
         # one packed buffer per net (every tensor starts on a 16-byte boundary), parameters as views: the update kernels
@@ -56,11 +52,11 @@ class _Net:
         p, n = self.p, x.shape[0]
         a, b = work
         w, bb, lw, lb = self.blocks[0]
-        _launch("spo_ma_mlp_layer", L.ptr(x), n, self.D, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), self.H,
-                L.ptr(p["base.feature_norm.weight"]), L.ptr(p["base.feature_norm.bias"]), L.ptr(a), L.stream())
+        L.call("spo_ma_mlp_layer", L.ptr(x), n, self.D, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), self.H,
+               L.ptr(p["base.feature_norm.weight"]), L.ptr(p["base.feature_norm.bias"]), L.ptr(a), L.stream())
         for w, bb, lw, lb in self.blocks[1:]:
-            _launch("spo_ma_mlp_layer", L.ptr(a), n, self.H, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), self.H, None, None,
-                    L.ptr(b), L.stream())
+            L.call("spo_ma_mlp_layer", L.ptr(a), n, self.H, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), self.H, None, None,
+                   L.ptr(b), L.stream())
             a, b = b, a
         return a
 
@@ -92,8 +88,8 @@ class MultiAgentNets:
         n = cent_obs.shape[0]
         feat = net.features(cent_obs, self._buffers(n, net.H))
         out = torch.empty(n, 1, dtype=torch.float32, device=self.device)
-        _launch("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["v_out.weight"]), L.ptr(net.p["v_out.bias"]), 1, None, 1.0, 1.0, None,
-                L.ptr(out), None, L.stream())
+        L.call("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["v_out.weight"]), L.ptr(net.p["v_out.bias"]), 1, None, 1.0, 1.0, None,
+               L.ptr(out), None, L.stream())
         return out
 
     def get_actions(self, cent_obs, obs, eps=None, deterministic=False):
@@ -110,9 +106,9 @@ class MultiAgentNets:
             eps = torch.randn(n, A, dtype=torch.float32, device=self.device)
         actions = torch.empty(n, A, dtype=torch.float32, device=self.device)
         logp = torch.empty(n, A, dtype=torch.float32, device=self.device)
-        _launch("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["act.action_out.fc_mean.weight"]), L.ptr(net.p["act.action_out.fc_mean.bias"]),
-                A, L.ptr(net.p["act.action_out.log_std"]), self.std_x_coef, self.std_y_coef, L.ptr(eps), L.ptr(actions),
-                L.ptr(logp), L.stream())
+        L.call("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["act.action_out.fc_mean.weight"]), L.ptr(net.p["act.action_out.fc_mean.bias"]),
+               A, L.ptr(net.p["act.action_out.log_std"]), self.std_x_coef, self.std_y_coef, L.ptr(eps), L.ptr(actions),
+               L.ptr(logp), L.stream())
         return self._value(self.critic, cent_obs), actions, logp, self._value(self.cost_critic, cent_obs)
 
 
@@ -123,8 +119,8 @@ class MultiAgentNets:
         n, A, net = obs.shape[0], self.act_dim, self.actor
         feat = net.features(obs, self._buffers(n, net.H))
         mean = torch.empty(n, A, dtype=torch.float32, device=self.device)
-        _launch("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["act.action_out.fc_mean.weight"]), L.ptr(net.p["act.action_out.fc_mean.bias"]),
-                A, L.ptr(net.p["act.action_out.log_std"]), self.std_x_coef, self.std_y_coef, None, L.ptr(mean), None, L.stream())
+        L.call("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(net.p["act.action_out.fc_mean.weight"]), L.ptr(net.p["act.action_out.fc_mean.bias"]),
+               A, L.ptr(net.p["act.action_out.log_std"]), self.std_x_coef, self.std_y_coef, None, L.ptr(mean), None, L.stream())
         std = torch.sigmoid(net.p["act.action_out.log_std"] / self.std_x_coef) * self.std_y_coef
         return -((actions - mean) ** 2) / (2 * std ** 2) - std.log() - _LOG_SQRT_2PI
 
@@ -172,12 +168,12 @@ class MultiAgentTrainer:
     def _forward_train(self, net, x, ws):
         p, n = net.p, x.shape[0]
         w, bb, lw, lb = net.blocks[0]
-        _launch("spo_ma_mlp_layer_train", L.ptr(x), n, net.D, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), net.H,
-                L.ptr(p["base.feature_norm.weight"]), L.ptr(p["base.feature_norm.bias"]), L.ptr(ws["out"][0]), L.ptr(ws["pre"][0]),
-                L.ptr(ws["xn"]), L.stream())
+        L.call("spo_ma_mlp_layer_train", L.ptr(x), n, net.D, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), net.H,
+               L.ptr(p["base.feature_norm.weight"]), L.ptr(p["base.feature_norm.bias"]), L.ptr(ws["out"][0]), L.ptr(ws["pre"][0]),
+               L.ptr(ws["xn"]), L.stream())
         for i, (w, bb, lw, lb) in enumerate(net.blocks[1:], start=1):
-            _launch("spo_ma_mlp_layer_train", L.ptr(ws["out"][i - 1]), n, net.H, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), net.H,
-                    None, None, L.ptr(ws["out"][i]), L.ptr(ws["pre"][i]), None, L.stream())
+            L.call("spo_ma_mlp_layer_train", L.ptr(ws["out"][i - 1]), n, net.H, L.ptr(p[w]), L.ptr(p[bb]), L.ptr(p[lw]), L.ptr(p[lb]), net.H,
+                   None, None, L.ptr(ws["out"][i]), L.ptr(ws["pre"][i]), None, L.stream())
         return ws["out"][-1]
 
     def _gemm_tn(self, A_, B_, out, R, M, N, ws):
@@ -186,8 +182,8 @@ class MultiAgentTrainer:
         slices = max(1, min(32, (296 + tiles - 1) // tiles, R // 256))
         while slices > 1 and (slices - 1) * (((R + slices - 1) // slices + 31) // 32 * 32) >= R:   # no empty slice (32-row chunks)
             slices -= 1
-        _launch("spo_ma_gemm_tn", L.ptr(A_), L.ptr(B_), L.ptr(ws["part"]), R, M, N, slices, L.stream())
-        _launch("spo_ma_partial_reduce", L.ptr(ws["part"]), slices, M * N, 1, M * N, L.ptr(out), None, None, 1.0, L.stream())
+        L.call("spo_ma_gemm_tn", L.ptr(A_), L.ptr(B_), L.ptr(ws["part"]), R, M, N, slices, L.stream())
+        L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), slices, M * N, 1, M * N, L.ptr(out), None, None, 1.0, L.stream())
 
     def _backward(self, net, x, ws, dfeat):
         """Gradients of every block and of the input LayerNorm from dfeat = d loss / d features (in ws['dy'])."""
@@ -196,42 +192,42 @@ class MultiAgentTrainer:
         dy, dy2 = dfeat, (ws["dy2"] if dfeat is ws["dy"] else ws["dy"])
         for i in reversed(range(len(net.blocks))):
             w, bb, lw, lb = net.blocks[i]
-            _launch("spo_ma_ln_elu_bwd", L.ptr(dy), L.ptr(ws["pre"][i]), L.ptr(p[lw]), n, H, L.ptr(ws["dz"]), L.ptr(ws["part"]), L.stream())
-            _launch("spo_ma_partial_reduce", L.ptr(ws["part"]), nb32, 3 * H, 3, H, L.ptr(g[lw]), L.ptr(g[lb]), L.ptr(g[bb]), 1.0, L.stream())
+            L.call("spo_ma_ln_elu_bwd", L.ptr(dy), L.ptr(ws["pre"][i]), L.ptr(p[lw]), n, H, L.ptr(ws["dz"]), L.ptr(ws["part"]), L.stream())
+            L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), nb32, 3 * H, 3, H, L.ptr(g[lw]), L.ptr(g[lb]), L.ptr(g[bb]), 1.0, L.stream())
             inp, K = (ws["out"][i - 1], H) if i > 0 else (ws["xn"], net.D)
             self._gemm_tn(ws["dz"], inp, g[w], n, H, K, ws)
-            _launch("spo_ma_gemm_nn", L.ptr(ws["dz"]), L.ptr(p[w]), L.ptr(dy2), n, K, H, L.stream())
+            L.call("spo_ma_gemm_nn", L.ptr(ws["dz"]), L.ptr(p[w]), L.ptr(dy2), n, K, H, L.stream())
             dy, dy2 = dy2, dy
-        _launch("spo_ma_ln_in_bwd", L.ptr(dy), L.ptr(x), n, net.D, L.ptr(ws["part"]), L.stream())
-        _launch("spo_ma_partial_reduce", L.ptr(ws["part"]), nb32, 2 * net.D, 2, net.D, L.ptr(g["base.feature_norm.weight"]),
-                L.ptr(g["base.feature_norm.bias"]), None, 1.0, L.stream())
+        L.call("spo_ma_ln_in_bwd", L.ptr(dy), L.ptr(x), n, net.D, L.ptr(ws["part"]), L.stream())
+        L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), nb32, 2 * net.D, 2, net.D, L.ptr(g["base.feature_norm.weight"]),
+               L.ptr(g["base.feature_norm.bias"]), None, 1.0, L.stream())
 
     def _clip_adam(self, net, lr):
         c = self.cfg
         net.step += 1
         norm = torch.empty(2, dtype=torch.float32, device=self.device)
-        _launch("spo_ma_clip_adam", L.ptr(net.flat), L.ptr(net.gflat), L.ptr(net.exp_avg), L.ptr(net.exp_avg_sq), net.flat.numel(),
-                float(c["max_grad_norm"]), float(lr), 0.9, 0.999, float(c["opti_eps"]), float(c["weight_decay"]), net.step,
-                L.ptr(self._adam_work), L.ptr(norm), L.stream())
+        L.call("spo_ma_clip_adam", L.ptr(net.flat), L.ptr(net.gflat), L.ptr(net.exp_avg), L.ptr(net.exp_avg_sq), net.flat.numel(),
+               float(c["max_grad_norm"]), float(lr), 0.9, 0.999, float(c["opti_eps"]), float(c["weight_decay"]), net.step,
+               L.ptr(self._adam_work), L.ptr(norm), L.stream())
         return norm[0]
 
     def _critic_update(self, net, share_obs, value_preds, returns, ws):
         """cal_value_loss (mappolag.py:121-133) + the critic's optimiser step (:174-186); returns (loss, grad norm)."""
         c, n, H = self.cfg, share_obs.shape[0], net.H
         feat = self._forward_train(net, share_obs, ws)
-        _launch("spo_ma_head", L.ptr(feat), n, H, L.ptr(net.p["v_out.weight"]), L.ptr(net.p["v_out.bias"]), 1, None, 1.0, 1.0, None,
-                L.ptr(ws["v"]), None, L.stream())
+        L.call("spo_ma_head", L.ptr(feat), n, H, L.ptr(net.p["v_out.weight"]), L.ptr(net.p["v_out.bias"]), 1, None, 1.0, 1.0, None,
+               L.ptr(ws["v"]), None, L.stream())
         # the reference normalises the returns twice, UPDATING the shared statistics both times: first for the clipped error
         for dst in (ws["rn_c"], ws["rn_o"]):
-            _launch("spo_ma_popart_normalize", L.ptr(returns), n, L.ptr(self.popart_state), self.popart_beta, self.popart_eps, L.ptr(dst), L.stream())
+            L.call("spo_ma_popart_normalize", L.ptr(returns), n, L.ptr(self.popart_state), self.popart_beta, self.popart_eps, L.ptr(dst), L.stream())
         nb256 = (n + 255) // 256
-        _launch("spo_ma_value_loss", L.ptr(ws["v"]), L.ptr(value_preds), L.ptr(ws["rn_c"]), L.ptr(ws["rn_o"]), n, float(c["clip_param"]),
-                float(c["huber_delta"]), float(c["value_loss_coef"]) / n, L.ptr(ws["dv"]), L.ptr(ws["part"]), L.stream())
+        L.call("spo_ma_value_loss", L.ptr(ws["v"]), L.ptr(value_preds), L.ptr(ws["rn_c"]), L.ptr(ws["rn_o"]), n, float(c["clip_param"]),
+               float(c["huber_delta"]), float(c["value_loss_coef"]) / n, L.ptr(ws["dv"]), L.ptr(ws["part"]), L.stream())
         loss = torch.empty(1, dtype=torch.float32, device=self.device)
-        _launch("spo_ma_partial_reduce", L.ptr(ws["part"]), nb256, 2, 1, 1, L.ptr(loss), None, None, 1.0 / n, L.stream())
-        _launch("spo_ma_partial_reduce", L.ptr(ws["part"]), nb256, 2, 2, 1, None, L.ptr(net.g["v_out.bias"]), None, 1.0, L.stream())
+        L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), nb256, 2, 1, 1, L.ptr(loss), None, None, 1.0 / n, L.stream())
+        L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), nb256, 2, 2, 1, None, L.ptr(net.g["v_out.bias"]), None, 1.0, L.stream())
         self._gemm_tn(ws["dv"], feat, net.g["v_out.weight"], n, 1, H, ws)
-        _launch("spo_ma_gemm_nn", L.ptr(ws["dv"]), L.ptr(net.p["v_out.weight"]), L.ptr(ws["dy"]), n, H, 1, L.stream())
+        L.call("spo_ma_gemm_nn", L.ptr(ws["dv"]), L.ptr(net.p["v_out.weight"]), L.ptr(ws["dy"]), n, H, 1, L.stream())
         self._backward(net, share_obs, ws, ws["dy"])
         return loss[0], self._clip_adam(net, c["critic_lr"])
 
@@ -262,19 +258,19 @@ class MultiAgentTrainer:
         nb32 = (n + 31) // 32
         imp = torch.empty(n, 1, dtype=torch.float32, device=dev)
         wm, bm, ls = net.p["act.action_out.fc_mean.weight"], net.p["act.action_out.fc_mean.bias"], net.p["act.action_out.log_std"]
-        _launch("spo_ma_actor_loss", L.ptr(feat), n, net.H, L.ptr(wm), L.ptr(bm), L.ptr(ls), A, L.ptr(actions), L.ptr(old_logp), L.ptr(adv),
-                L.ptr(cost_adv), L.ptr(factor), L.ptr(self.lamda_lagr), 1.0 - float(c["clip_param"]), 1.0 + float(c["clip_param"]),
-                nets.std_x_coef, nets.std_y_coef, L.ptr(ws["dmean"]), L.ptr(imp), L.ptr(ws["part"]), L.stream())
+        L.call("spo_ma_actor_loss", L.ptr(feat), n, net.H, L.ptr(wm), L.ptr(bm), L.ptr(ls), A, L.ptr(actions), L.ptr(old_logp), L.ptr(adv),
+               L.ptr(cost_adv), L.ptr(factor), L.ptr(self.lamda_lagr), 1.0 - float(c["clip_param"]), 1.0 + float(c["clip_param"]),
+               nets.std_x_coef, nets.std_y_coef, L.ptr(ws["dmean"]), L.ptr(imp), L.ptr(ws["part"]), L.stream())
         scal = torch.empty(2, dtype=torch.float32, device=dev)
-        _launch("spo_ma_actor_finalize", L.ptr(ws["part"]), nb32, n, L.ptr(ls), A, nets.std_x_coef, nets.std_y_coef, float(c["entropy_coef"]),
-                L.ptr(net.g["act.action_out.fc_mean.bias"]), L.ptr(net.g["act.action_out.log_std"]), L.ptr(scal), L.stream())
+        L.call("spo_ma_actor_finalize", L.ptr(ws["part"]), nb32, n, L.ptr(ls), A, nets.std_x_coef, nets.std_y_coef, float(c["entropy_coef"]),
+               L.ptr(net.g["act.action_out.fc_mean.bias"]), L.ptr(net.g["act.action_out.log_std"]), L.ptr(scal), L.stream())
         self._gemm_tn(ws["dmean"], feat, net.g["act.action_out.fc_mean.weight"], n, A, net.H, ws)
-        _launch("spo_ma_gemm_nn", L.ptr(ws["dmean"]), L.ptr(wm), L.ptr(ws["dy"]), n, net.H, A, L.stream())
+        L.call("spo_ma_gemm_nn", L.ptr(ws["dmean"]), L.ptr(wm), L.ptr(ws["dy"]), n, net.H, A, L.stream())
         self._backward(net, obs, ws, ws["dy"])
         actor_grad_norm = self._clip_adam(net, c["actor_lr"])
         # ---- Lagrange multiplier (uses the importance weights of THIS update, mappolag.py:169-172) ----
-        _launch("spo_ma_lagrange_step", L.ptr(imp), L.ptr(cost_adv), L.ptr(aver_costs), n, float(c["cost_limit"]), float(c["gamma"]),
-                float(c["lagrangian_coef_rate"]), L.ptr(self.lamda_lagr), L.stream())
+        L.call("spo_ma_lagrange_step", L.ptr(imp), L.ptr(cost_adv), L.ptr(aver_costs), n, float(c["cost_limit"]), float(c["gamma"]),
+               float(c["lagrangian_coef_rate"]), L.ptr(self.lamda_lagr), L.stream())
         # ---- critics ----
         value_loss, critic_grad_norm = self._critic_update(nets.critic, share_obs, value_preds, returns, self._ws(n, nets.critic))
         cost_loss, cost_grad_norm = self._critic_update(nets.cost_critic, share_obs, cost_preds, cost_returns, self._ws(n, nets.cost_critic))

@@ -114,7 +114,6 @@ class ActorVCritic(nn.Module):
         if device.type != "cuda":
             self.flat = None
             return
-        lib = L.lib()
         self.n_actor, self.n_critic, self.n_total = L.param_count(self.dims)
         flat = torch.empty(self.n_total, dtype=torch.float32, device=device)
         off = 0
@@ -175,10 +174,9 @@ class ActorVCritic(nn.Module):
             self._philox_seed = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF
         self._philox_offset += 1
         st, t = (C.byref(store[0]), int(store[1])) if store is not None else (None, 0)
-        L.check(L.lib().spo_policy_step(C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), L.ptr(eps),
-                                        self._philox_seed, self._philox_offset, int(bool(deterministic)), n,
-                                        L.ptr(act), L.ptr(logp), L.ptr(v_r), L.ptr(v_c), st, t, L.stream()),
-                "spo_policy_step")
+        L.call("spo_policy_step", C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), L.ptr(eps),
+               self._philox_seed, self._philox_offset, int(bool(deterministic)), n,
+               L.ptr(act), L.ptr(logp), L.ptr(v_r), L.ptr(v_c), st, t, L.stream())
         if act is None:
             return None
         if single:
@@ -190,16 +188,15 @@ class ActorVCritic(nn.Module):
         n = o2.shape[0]
         v_r = torch.empty(n, dtype=torch.float32, device=o2.device)
         v_c = torch.empty(n, dtype=torch.float32, device=o2.device)
-        L.check(L.lib().spo_critic_values(C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), n, L.ptr(v_r), L.ptr(v_c),
-                                          L.stream()), "spo_critic_values")
+        L.call("spo_critic_values", C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), n, L.ptr(v_r), L.ptr(v_c),
+               L.stream())
         return (v_r[0], v_c[0]) if single else (v_r, v_c)
 
     def actor_mean(self, obs):
         o2, single = self._check(obs)
         n = o2.shape[0]
         mean = torch.empty(n, self.act_dim, dtype=torch.float32, device=o2.device)
-        L.check(L.lib().spo_actor_forward(C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), n, L.ptr(mean), L.stream()),
-                "spo_actor_forward")
+        L.call("spo_actor_forward", C.byref(self.dims), L.ptr(self.flat), L.ptr(o2), n, L.ptr(mean), L.stream())
         return mean[0] if single else mean
 
     def forward(self, obs):

@@ -77,9 +77,8 @@ class SafeNormalizeObservation:
         n = obs.shape[0]
         if out is None:
             out = torch.empty_like(obs)
-        L.check(L.lib().spo_obs_normalize(L.ptr(obs), n, self.obs_dim, L.ptr(self.obs_rms.mean), L.ptr(self.obs_rms.var),
-                                          self.obs_rms.count, None, 1 if update else 0, self.epsilon, L.ptr(out), L.stream()),
-                "spo_obs_normalize")
+        L.call("spo_obs_normalize", L.ptr(obs), n, self.obs_dim, L.ptr(self.obs_rms.mean), L.ptr(self.obs_rms.var),
+               self.obs_rms.count, None, 1 if update else 0, self.epsilon, L.ptr(out), L.stream())
         if update:
             self.obs_rms.count += n
         return out
@@ -102,6 +101,6 @@ class SafeRescaleAction:
             raise L.SpoError(f"act must be fp32 [n, {A}], got {tuple(act.shape)} {act.dtype}")
         if out is None:
             out = torch.empty_like(act)
-        L.check(L.lib().spo_action_rescale(L.ptr(act), act.shape[0], A, L.ptr(self.low), L.ptr(self.high), self.min_action,
-                                           self.max_action, L.ptr(out), L.stream()), "spo_action_rescale")
+        L.call("spo_action_rescale", L.ptr(act), act.shape[0], A, L.ptr(self.low), L.ptr(self.high), self.min_action,
+               self.max_action, L.ptr(out), L.stream())
         return out

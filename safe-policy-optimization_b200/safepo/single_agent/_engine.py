@@ -1,4 +1,4 @@
-"""Shared machinery of the four single-agent trainers (ppo_lag, focops, cpo, trpo_lag).
+"""Shared machinery of the twelve single-agent trainers (ppo_lag, focops, cpo, trpo_lag and their siblings).
 
 What the reference spells out four times as python loops
 (safepo/single_agent/ppo_lag.py:159-349 and the byte-identical rollout blocks of
@@ -34,6 +34,35 @@ from safepo.common.buffer import VectorizedOnPolicyBuffer
 from safepo.common.lagrange import Lagrange, PIDLagrangian
 from safepo.common.logger import EpochLogger
 from safepo.common.model import ActorVCritic
+
+CUP_LAMBDA, CUP_NU = 0.95, 0.20       # cup.py:45-46
+
+
+def _lagrange(upper_bound=None):
+    return lambda args: Lagrange(args.cost_limit, args.lagrangian_multiplier_init, args.lagrangian_multiplier_lr,
+                                 lagrangian_upper_bound=upper_bound)
+
+
+# What sets the algorithms of a family apart.  Policy-gradient family (ppo_lag.py and its siblings, SURVEY 8f rank 2):
+# algorithm -> (loss kind of spo_pg_update, multiplier factory or None).
+PG_ALGOS = {
+    "ppo_lag": (L.LOSS_PPO_CLIP, _lagrange()),
+    "ppo": (L.LOSS_PPO_CLIP, None),
+    "pg": (L.LOSS_PG, None),
+    "cppo_pid": (L.LOSS_PPO_CLIP, lambda args: PIDLagrangian(args.cost_limit, args.lagrangian_multiplier_init)),
+    "cup": (L.LOSS_PPO_CLIP, _lagrange(CUP_NU)),
+    "focops": (L.LOSS_FOCOPS, _lagrange(2.0)),
+}
+# Trust-region family (cpo.py, trpo_lag.py and their siblings): algorithm -> (TrustRegionUpdate step: run_cpo with this
+# variant, run_trpo or run_npg; multiplier factory or None; whether Misc/AcceptanceStep is logged).
+TR_ALGOS = {
+    "cpo": ("cpo", None, True),
+    "pcpo": ("pcpo", None, True),
+    "trpo_lag": ("trpo", _lagrange(), True),
+    "trpo": ("trpo", None, True),
+    "rcpo": ("npg", _lagrange(), False),
+    "natural_pg": ("npg", None, False),
+}
 
 
 # ---------------------------------------------------------------------------------------
@@ -82,7 +111,7 @@ class AdamState:
         self.t = torch.zeros(3, dtype=torch.int32, device=dev)
 
 
-def _normalizer_state(roll, env):
+def _normalizer_state(roll):
     """What the reference checkpoints as "Normalizer" (ppo_lag.py:381-386: env.obs_rms): a host object with ``mean`` / ``var`` /
     ``count`` numpy fields and ``update()`` like gymnasium's RunningMeanStd -- evaluate.py:56-57 assigns the unpickled object
     straight to ``eval_env.obs_rms`` -- holding the device-side statistics when observations are normalised on the device, else
@@ -90,7 +119,7 @@ def _normalizer_state(roll, env):
     norm = getattr(roll, "obs_norm", None)
     if norm is not None:
         return norm.obs_rms.host_copy()
-    return getattr(env, "obs_rms", None)
+    return getattr(roll.env, "obs_rms", None)
 
 
 def make_ctrl(device):
@@ -302,26 +331,65 @@ class DeviceTapeRollout(Rollout):
 
 
 # ---------------------------------------------------------------------------------------
-# PPO-Lag / FOCOPS update
+# minibatch updates: PPO-Lag / FOCOPS actor + critics, CPO / TRPO-Lag critics
 # ---------------------------------------------------------------------------------------
 
-class PolicyGradientUpdate:
-    def __init__(self, policy, cfg, kind, epochs, host_rng, device, focops_lam=1.5, dp=None):
-        self.policy, self.cfg, self.kind, self.host_rng, self.device = policy, cfg, kind, host_rng, device
+def _old_dist(policy, obs, old_mean, old_log_std):
+    """The old distribution of ppo_lag.py:277 / cpo.py:365: the actor's mean on ``obs`` into ``old_mean`` (reallocated when
+    the batch size changed) and its log_std into ``old_log_std``.  Returns old_mean."""
+    S = obs.shape[0]
+    if old_mean is None or old_mean.shape[0] != S:
+        old_mean = torch.empty(S, policy.act_dim, dtype=torch.float32, device=old_log_std.device)
+    L.call("spo_actor_forward", C.byref(policy.dims), L.ptr(policy.flat), L.ptr(obs), S, L.ptr(old_mean), L.stream())
+    old_log_std.copy_(policy.flat[: policy.act_dim])
+    return old_mean
+
+
+class _MinibatchUpdate:
+    """What PolicyGradientUpdate and CriticRegression share: Adam state, control block and hyper-parameters of
+    ``spo_pg_update``, and one pass of it over a shuffled batch."""
+
+    def __init__(self, policy, cfg, host_rng, device, dp, lr_actor, lr_critic, focops_lam, focops_kl):
+        self.policy, self.cfg, self.host_rng, self.device = policy, cfg, host_rng, device
         self.dp = dp          # safepo.common.dist.DataParallel or None
+        self.adam = AdamState(policy)
+        self.ctrl = make_ctrl(device)
+        self.hp = L.HParams(lr_actor, lr_critic, lr_critic, 0.9, 0.999, 1e-8, cfg["max_grad_norm"],
+                            0.001 if cfg.get("use_critic_norm", True) else 0.0, 0.8, 1.2, focops_lam, focops_kl,
+                            2.0 if cfg.get("use_value_coefficient", False) else 1.0)
+
+    def _pass(self, it, batch, kind, perms):
+        """Pass ``it`` over ``batch`` in one persistent launch, in the order perms[it] if given, else the reference's
+        DataLoader order (host RNG) or a device permutation."""
+        S, B = batch.count, self.cfg["batch_size"]
+        if perms is not None:
+            perm = perms[it].to(self.device)
+        elif self.host_rng:
+            perm = reference_order(S).to(self.device)
+        else:
+            perm = torch.randperm(S, device=self.device)
+        pol, adam = self.policy, self.adam
+        args = (C.byref(pol.dims), L.ptr(pol.flat), L.ptr(adam.m), L.ptr(adam.v), L.ptr(adam.t), C.byref(batch), L.ptr(perm),
+                perm.numel(), B, kind, C.byref(self.hp), L.ptr(self.ctrl))
+        if self.dp is None:
+            L.call("spo_pg_update", *args, L.stream())
+        else:
+            # ranks hold equal-sized shards; gradients are summed inside the kernel over NVLink
+            comm = self.dp.comm_struct()
+            L.call("spo_pg_update_dp", *args, C.byref(comm), L.stream())
+            self.dp.advance((perm.numel() + B - 1) // B)
+
+
+class PolicyGradientUpdate(_MinibatchUpdate):
+    def __init__(self, policy, cfg, kind, epochs, host_rng, device, focops_lam=1.5, dp=None):
         if dp is not None:
             dp.broadcast(policy.flat)
             dp.setup_peer_buffers(policy.dims, device)
-        self.adam = AdamState(policy)
+        super().__init__(policy, cfg, host_rng, device, dp, 3e-4, 3e-4, focops_lam, cfg["target_kl"])
+        self.kind = kind
         self.sched = LinearDecay(3e-4, epochs)
-        self.ctrl = make_ctrl(device)
-        self.hp = L.HParams(3e-4, 3e-4, 3e-4, 0.9, 0.999, 1e-8, cfg["max_grad_norm"],
-                            0.001 if cfg.get("use_critic_norm", True) else 0.0, 0.8, 1.2, focops_lam, cfg["target_kl"],
-                            2.0 if cfg.get("use_value_coefficient", False) else 1.0)
         self.old_mean = None
         self.old_log_std = torch.zeros(policy.act_dim, dtype=torch.float32, device=device)
-        self.old_std_full = None
-        self.launches = 0
 
     def run(self, data, perms=None, refresh_old=True, kind=None, cup_coef=None, step_sched=True):
         """data: dict from buffer.get(lam).  Returns dict(stop_iter, kl, losses(3)).
@@ -329,20 +397,14 @@ class PolicyGradientUpdate:
         loop one minibatch at a time).  kind / cup_coef: run this call with another loss kind on the same
         optimizer state (CUP's projection stage, cup.py:355-404); step_sched=False leaves the actor's
         LinearLR alone (it steps once per epoch, after both stages)."""
-        pol, cfg, lib = self.policy, self.cfg, L.lib()
+        pol, cfg = self.policy, self.cfg
         kind = self.kind if kind is None else kind
         focops_lam_saved = self.hp.focops_lam
         if kind == L.LOSS_CUP_PROJECTION:
             self.hp.focops_lam = float(cup_coef)
         S = data["obs"].shape[0]
-        d = pol.dims
-        if self.old_mean is None or self.old_mean.shape[0] != S:
-            self.old_mean = torch.empty(S, pol.act_dim, dtype=torch.float32, device=self.device)
-            refresh_old = True
-        if refresh_old:
-            L.check(lib.spo_actor_forward(C.byref(d), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(self.old_mean), L.stream()),
-                    "spo_actor_forward")
-            self.old_log_std.copy_(pol.flat[: pol.act_dim])
+        if refresh_old or self.old_mean is None or self.old_mean.shape[0] != S:
+            self.old_mean = _old_dist(pol, data["obs"], self.old_mean, self.old_log_std)
         old_std = None
         if kind in (L.LOSS_FOCOPS, L.LOSS_CUP_PROJECTION):
             old_std = torch.exp(self.old_log_std).expand(S, pol.act_dim).contiguous()
@@ -350,37 +412,17 @@ class PolicyGradientUpdate:
                         L.ptr(data["target_value_c"]), L.ptr(data["adv"]), L.ptr(self.old_mean), L.ptr(old_std), S)
         self.hp.lr_actor = self.sched.lr
         self.ctrl.zero_()
-        self.launches += 3
         for it in range(cfg["learning_iters"]):
-            if perms is not None:
-                perm = perms[it].to(self.device)
-            elif self.host_rng:
-                perm = reference_order(S).to(self.device)
-            else:
-                perm = torch.randperm(S, device=self.device)
+            self._pass(it, batch, kind, perms)
             if self.dp is None:
-                L.check(lib.spo_pg_update(C.byref(d), L.ptr(pol.flat), L.ptr(self.adam.m), L.ptr(self.adam.v), L.ptr(self.adam.t),
-                                          C.byref(batch), L.ptr(perm), perm.numel(), cfg["batch_size"], kind, C.byref(self.hp),
-                                          L.ptr(self.ctrl), L.stream()), "spo_pg_update")
-                L.check(lib.spo_actor_kl(C.byref(d), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(self.old_mean),
-                                         L.ptr(self.old_log_std), S, 0, cfg["target_kl"], L.ptr(self.ctrl), L.stream()),
-                        "spo_actor_kl")
+                L.call("spo_actor_kl", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(self.old_mean),
+                       L.ptr(self.old_log_std), S, 0, cfg["target_kl"], L.ptr(self.ctrl), L.stream())
             else:
-                # ranks hold equal-sized shards; gradients are summed inside the kernel over NVLink
-                comm = self.dp.comm_struct()
-                L.check(lib.spo_pg_update_dp(C.byref(d), L.ptr(pol.flat), L.ptr(self.adam.m), L.ptr(self.adam.v),
-                                             L.ptr(self.adam.t), C.byref(batch), L.ptr(perm), perm.numel(), cfg["batch_size"],
-                                             kind, C.byref(self.hp), L.ptr(self.ctrl), C.byref(comm), L.stream()),
-                        "spo_pg_update_dp")
-                self.dp.advance((perm.numel() + cfg["batch_size"] - 1) // cfg["batch_size"])
-                L.check(lib.spo_actor_kl_accumulate(C.byref(d), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(self.old_mean),
-                                                    L.ptr(self.old_log_std), S, L.ptr(self.ctrl), L.stream()),
-                        "spo_actor_kl_accumulate")
+                L.call("spo_actor_kl_accumulate", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(self.old_mean),
+                       L.ptr(self.old_log_std), S, L.ptr(self.ctrl), L.stream())
                 kl_sum = self.ctrl.view(torch.float64)[L.CTRL_KL_SUM_F64_INDEX:L.CTRL_KL_SUM_F64_INDEX + 1]
                 self.dp.all_reduce_sum(kl_sum)
-                L.check(lib.spo_kl_finalize(L.ptr(self.ctrl), float(S * self.dp.world), cfg["target_kl"], L.stream()),
-                        "spo_kl_finalize")
-            self.launches += 2
+                L.call("spo_kl_finalize", L.ptr(self.ctrl), float(S * self.dp.world), cfg["target_kl"], L.stream())
             if self.host_rng or perms is not None:
                 # the reference stops drawing permutations once KL trips: stay in lock-step with its RNG
                 if int(read_ctrl(self.ctrl)["stop"]):
@@ -395,11 +437,7 @@ class PolicyGradientUpdate:
                 "steps": int(c["steps"])}
 
 
-# ---------------------------------------------------------------------------------------
-# CPO / TRPO-Lag update
-# ---------------------------------------------------------------------------------------
-
-class CriticRegression:
+class CriticRegression(_MinibatchUpdate):
     """cpo.py:534-571 / trpo_lag.py:457-494: minibatch regression of the two critics
     (batch 128, lr 1e-3, 10 passes).  The joint clip (cpo.py:562) runs over policy.parameters(), but
     every fvp() call starts with policy.actor.zero_grad() (cpo.py:137, trpo_lag.py:139), which sets the
@@ -408,44 +446,26 @@ class CriticRegression:
     caller whose actor does hold a gradient at this point."""
 
     def __init__(self, policy, cfg, host_rng, device, lr=1e-3, dp=None):
-        self.policy, self.cfg, self.host_rng, self.device, self.dp = policy, cfg, host_rng, device, dp
         if dp is not None and dp._peer is None:
             dp.setup_peer_buffers(policy.dims, device)
-        self.adam = AdamState(policy)
-        self.ctrl = make_ctrl(device)
-        self.hp = L.HParams(0.0, lr, lr, 0.9, 0.999, 1e-8, cfg["max_grad_norm"],
-                            0.001 if cfg.get("use_critic_norm", True) else 0.0, 0.8, 1.2, 1.5, 0.0,
-                            2.0 if cfg.get("use_value_coefficient", False) else 1.0)
+        super().__init__(policy, cfg, host_rng, device, dp, 0.0, lr, 1.5, 0.0)
 
     def run(self, data, stale_actor_grad_sumsq=0.0, perms=None):
-        pol, cfg, lib = self.policy, self.cfg, L.lib()
         S = data["obs"].shape[0]
         batch = L.Batch(L.ptr(data["obs"]), None, None, L.ptr(data["target_value_r"]), L.ptr(data["target_value_c"]),
                         None, None, None, S)
         self.ctrl.zero_()
         self.ctrl.view(torch.float32)[L.CTRL_EXTRA_SUMSQ_F32_INDEX] = stale_actor_grad_sumsq
-        for it in range(cfg["learning_iters"]):
-            if perms is not None:
-                perm = perms[it].to(self.device)
-            elif self.host_rng:
-                perm = reference_order(S).to(self.device)
-            else:
-                perm = torch.randperm(S, device=self.device)
-            if self.dp is None:
-                L.check(lib.spo_pg_update(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(self.adam.m), L.ptr(self.adam.v),
-                                          L.ptr(self.adam.t), C.byref(batch), L.ptr(perm), perm.numel(), cfg["batch_size"],
-                                          L.LOSS_CRITIC_ONLY, C.byref(self.hp), L.ptr(self.ctrl), L.stream()), "spo_pg_update")
-            else:       # per-rank batch, critic gradients summed inside the kernel over NVLink like the policy-gradient trainers
-                comm = self.dp.comm_struct()
-                L.check(lib.spo_pg_update_dp(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(self.adam.m), L.ptr(self.adam.v),
-                                             L.ptr(self.adam.t), C.byref(batch), L.ptr(perm), perm.numel(), cfg["batch_size"],
-                                             L.LOSS_CRITIC_ONLY, C.byref(self.hp), L.ptr(self.ctrl), C.byref(comm), L.stream()),
-                        "spo_pg_update_dp")
-                self.dp.advance((perm.numel() + cfg["batch_size"] - 1) // cfg["batch_size"])
+        for it in range(self.cfg["learning_iters"]):
+            self._pass(it, batch, L.LOSS_CRITIC_ONLY, perms)
         c = read_ctrl(self.ctrl)
         steps = max(int(c["steps"]), 1)
         return {"loss_r": c["loss_sum"][0] / steps, "loss_c": c["loss_sum"][1] / steps, "steps": int(c["steps"])}
 
+
+# ---------------------------------------------------------------------------------------
+# CPO / TRPO-Lag actor update
+# ---------------------------------------------------------------------------------------
 
 class TrustRegionUpdate:
     """Actor step of cpo.py:351-519 / trpo_lag.py:358-442 on the libspo kernels.  The flat
@@ -478,9 +498,8 @@ class TrustRegionUpdate:
     def _grad(self, data, adv, out):
         pol = self.policy
         S = data["obs"].shape[0]
-        L.check(L.lib().spo_surrogate_grad(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(data["act"]),
-                                           L.ptr(data["log_prob"]), L.ptr(adv), S, L.ptr(self.loss), L.ptr(out), L.stream()),
-                "spo_surrogate_grad")
+        L.call("spo_surrogate_grad", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(data["act"]),
+               L.ptr(data["log_prob"]), L.ptr(adv), S, L.ptr(self.loss), L.ptr(out), L.stream())
         if self.dp is not None:
             self.dp.all_reduce_mean(out)
             self.dp.all_reduce_mean(self.loss)
@@ -491,47 +510,72 @@ class TrustRegionUpdate:
         S = data["obs"].shape[0]
         if self.dp is not None:
             # the solver split at the FVP: p = work[P:2P] -> z = work[2P:3P], averaged over the ranks, then one CG step
-            lib, P = L.lib(), pol.n_actor
-            L.check(lib.spo_cg_begin(C.byref(pol.dims), L.ptr(rhs), L.ptr(out), L.ptr(self.work), L.stream()), "spo_cg_begin")
+            P = pol.n_actor
+            L.call("spo_cg_begin", C.byref(pol.dims), L.ptr(rhs), L.ptr(out), L.ptr(self.work), L.stream())
             p_vec, z_vec = self.work[P:2 * P], self.work[2 * P:3 * P]
             for _ in range(self.CG_ITERS):
-                L.check(lib.spo_fvp(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(p_vec), self.DAMPING,
-                                    L.ptr(z_vec), L.stream()), "spo_fvp")
+                L.call("spo_fvp", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(p_vec), self.DAMPING,
+                       L.ptr(z_vec), L.stream())
                 self.dp.all_reduce_mean(z_vec)
-                L.check(lib.spo_cg_update(C.byref(pol.dims), L.ptr(out), L.ptr(self.work), 1e-10, 1e-6, L.stream()), "spo_cg_update")
+                L.call("spo_cg_update", C.byref(pol.dims), L.ptr(out), L.ptr(self.work), 1e-10, 1e-6, L.stream())
             L.LAUNCHES["n"] += self.CG_ITERS + 1
             return
-        L.check(L.lib().spo_conjugate_gradient(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(rhs),
-                                               self.CG_ITERS, self.DAMPING, 1e-10, 1e-6, L.ptr(out), L.ptr(self.work),
-                                               L.stream()), "spo_conjugate_gradient")
+        L.call("spo_conjugate_gradient", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(rhs),
+               self.CG_ITERS, self.DAMPING, 1e-10, 1e-6, L.ptr(out), L.ptr(self.work), L.stream())
         L.LAUNCHES["n"] += 2 * self.CG_ITERS + 1
 
     def _fvp(self, data, v, out):
         pol = self.policy
         S = data["obs"].shape[0]
-        L.check(L.lib().spo_fvp(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(v), self.DAMPING, L.ptr(out),
-                                L.stream()), "spo_fvp")
+        L.call("spo_fvp", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(v), self.DAMPING, L.ptr(out),
+               L.stream())
         if self.dp is not None:
             self.dp.all_reduce_mean(out)
 
     def _eval(self, data, adv_a, adv_b):
         pol = self.policy
         S = data["obs"].shape[0]
-        L.check(L.lib().spo_linesearch_eval(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(data["act"]),
-                                            L.ptr(data["log_prob"]), L.ptr(adv_a), L.ptr(adv_b), L.ptr(self.old_mean),
-                                            L.ptr(self.old_log_std), S, L.ptr(self.out3), L.stream()), "spo_linesearch_eval")
+        L.call("spo_linesearch_eval", C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), L.ptr(data["act"]),
+               L.ptr(data["log_prob"]), L.ptr(adv_a), L.ptr(adv_b), L.ptr(self.old_mean), L.ptr(self.old_log_std), S,
+               L.ptr(self.out3), L.stream())
         if self.dp is not None:
             self.dp.all_reduce_mean(self.out3)
         return self.out3.cpu()
 
     def _old_dist(self, data):
-        pol = self.policy
-        S = data["obs"].shape[0]
-        if self.old_mean is None or self.old_mean.shape[0] != S:
-            self.old_mean = torch.empty(S, pol.act_dim, dtype=torch.float32, device=self.device)
-        L.check(L.lib().spo_actor_forward(C.byref(pol.dims), L.ptr(pol.flat), L.ptr(data["obs"]), S, L.ptr(self.old_mean),
-                                          L.stream()), "spo_actor_forward")
-        self.old_log_std.copy_(pol.flat[: pol.act_dim])
+        self.old_mean = _old_dist(self.policy, data["obs"], self.old_mean, self.old_log_std)
+
+    # -- the steps shared by CPO, TRPO and NPG --
+    def _direction(self, data, adv):
+        """theta_old, g = grad mean(ratio * adv), the old distribution, x = (F + damping I)^-1 g by conjugate gradient
+        and F x (cpo.py:353-372, trpo_lag.py:363-380).  Returns theta_old and the surrogate loss (device)."""
+        theta_old = self.policy.actor_flat().clone()
+        loss = self._grad(data, adv, self.g)
+        self._old_dist(data)
+        self._cg(data, self.g, self.x)
+        self._fvp(data, self.x, self.Fx)
+        return theta_old, loss
+
+    def _scalars(self, loss, *extra):
+        """The one device->host read of the update: [xHx, loss, |g|^2, |x|^2, *extra].  Returns them with the step
+        length alpha = sqrt(2 target_kl / xHx)."""
+        sc = torch.stack([torch.dot(self.x, self.Fx), loss[0], torch.dot(self.g, self.g), torch.dot(self.x, self.x),
+                          *extra]).cpu()
+        assert torch.isfinite(self.x).all(), "x is not finite"
+        assert sc[0].item() >= 0, "xHx is negative"
+        return sc, torch.sqrt(2 * self.cfg["target_kl"] / (sc[0] + 1e-8))
+
+    def _misc(self, sc, alpha, step):
+        return {"Misc/Alpha": alpha.item(), "Misc/FinalStepNorm": float(torch.norm(step)), "Misc/xHx": sc[0].item(),
+                "Misc/gradient_norm": float(sc[2].sqrt()), "Misc/H_inv_g": float(sc[3].sqrt())}
+
+    def _finish(self, theta_old, step, step_frac, acceptance, sc, alpha):
+        """End of a line search: apply step_frac * step, or return to theta_old if no step was accepted (acceptance 0)."""
+        if not acceptance:
+            self._log("INFO: no suitable step found...")
+            step = torch.zeros_like(step)
+        self.policy.actor_flat().copy_(theta_old + step_frac * step)
+        return {**self._misc(sc, alpha, step), "Misc/AcceptanceStep": acceptance}
 
     # -- CPO --
     def run_cpo(self, data, ep_costs, variant="cpo"):
@@ -539,21 +583,13 @@ class TrustRegionUpdate:
         variant="pcpo" (pcpo.py:371,392-401): projection step instead of the case analysis, optim_case 0,
         up to 200 line-search steps (pcpo.py:44)."""
         pol, kl_target = self.policy, self.cfg["target_kl"]
-        theta_old = pol.actor_flat().clone()
-        loss_r = self._grad(data, data["adv_r"], self.g)            # g = -grad(loss_pi_r) = grad mean(ratio*adv_r)
-        self._old_dist(data)
-        self._cg(data, self.g, self.x)
-        self._fvp(data, self.x, self.Fx)
+        theta_old, loss_r = self._direction(data, data["adv_r"])   # g = -grad(loss_pi_r) = grad mean(ratio*adv_r)
         loss_c = self._grad(data, data["adv_c"], self.b)            # b = grad mean(ratio*adv_c)
         self._cg(data, self.b, self.p)
-        sc = torch.stack([torch.dot(self.x, self.Fx), torch.dot(self.g, self.p), torch.dot(self.b, self.p),
-                          torch.dot(self.b, self.b), loss_r[0], loss_c[0], torch.dot(self.g, self.g),
-                          torch.dot(self.x, self.x)]).cpu()
-        xHx, r, s, bb = sc[0], sc[1], sc[2], sc[3]
-        loss_reward_before, loss_cost_before = -float(sc[4]), float(sc[5])
-        assert torch.isfinite(self.x).all(), "x is not finite"
-        assert xHx.item() >= 0, "xHx is negative"
-        alpha = torch.sqrt(2 * kl_target / (xHx + 1e-8))
+        sc, alpha = self._scalars(loss_r, torch.dot(self.g, self.p), torch.dot(self.b, self.p), torch.dot(self.b, self.b),
+                                  loss_c[0])
+        xHx, r, s, bb = sc[0], sc[4], sc[5], sc[6]
+        loss_reward_before, loss_cost_before = -float(sc[1]), float(sc[7])
         q = xHx
         search_steps = self.SEARCH_STEPS
         if variant == "pcpo":
@@ -599,11 +635,10 @@ class TrustRegionUpdate:
         else:
             lambda_star, nu_star = torch.zeros(1), torch.sqrt(2 * kl_target / (s + 1e-8))
             step = -nu_star.item() * self.p
-        step_frac, acceptance, accepted, kl = 1.0, 0, False, 0.0
+        step_frac, acceptance, kl = 1.0, 0, 0.0
         expected = float(torch.dot(self.g, step))
         for i in range(search_steps):
             pol.actor_flat().copy_(theta_old + step_frac * step)
-            acceptance = i + 1
             o = self._eval(data, data["adv_r"], data["adv_c"])
             loss_reward, loss_cost, kl = -float(o[0]), float(o[1]), float(o[2])
             improve, cost_diff = loss_reward_before - loss_reward, loss_cost - loss_cost_before
@@ -619,36 +654,22 @@ class TrustRegionUpdate:
                 self._log(f"INFO: violated KL constraint {kl} at step {i + 1}.")
             else:
                 self._log(f"Accept step at i={i + 1}")
-                accepted = True
+                acceptance = i + 1
                 break
             step_frac *= self.STEP_FRACTION
-        if not accepted:
-            self._log("INFO: no suitable step found...")
-            step = torch.zeros_like(step)
-            acceptance = 0
-        pol.actor_flat().copy_(theta_old + step_frac * step)
-        return {"Misc/Alpha": alpha.item(), "Misc/FinalStepNorm": float(torch.norm(step)), "Misc/xHx": xHx.item(),
-                "Misc/gradient_norm": float(sc[6].sqrt()), "Misc/H_inv_g": float(sc[7].sqrt()), "Misc/AcceptanceStep": acceptance,
-                "Loss/Loss_actor": -float(sc[4]) + float(sc[5]), "Train/KL": kl, "case": case, "step_frac": step_frac}
+        return {**self._finish(theta_old, step, step_frac, acceptance, sc, alpha),
+                "Loss/Loss_actor": loss_reward_before + loss_cost_before, "Train/KL": kl, "case": case, "step_frac": step_frac}
 
     # -- TRPO-Lag --
     def run_trpo(self, data, advantage):
         """trpo_lag.py:363-442."""
         pol, kl_target = self.policy, self.cfg["target_kl"]
-        theta_old = pol.actor_flat().clone()
-        loss0 = self._grad(data, advantage, self.g)
-        self._old_dist(data)
-        self._cg(data, self.g, self.x)
-        self._fvp(data, self.x, self.Fx)
-        sc = torch.stack([torch.dot(self.x, self.Fx), loss0[0], torch.dot(self.g, self.g), torch.dot(self.x, self.x)]).cpu()
-        xHx = sc[0]
+        theta_old, loss0 = self._direction(data, advantage)
+        sc, alpha = self._scalars(loss0)
         loss_before = -float(sc[1])
-        assert torch.isfinite(self.x).all(), "x is not finite"
-        assert xHx.item() >= 0, "xHx is negative"
-        alpha = torch.sqrt(2 * kl_target / (xHx + 1e-8))
         step = self.x * alpha.item()
         expected = float(torch.dot(self.g, step))
-        step_frac, final_kl, acceptance, accepted, loss_pi = 1.0, 0.0, 0, False, loss_before
+        step_frac, final_kl, acceptance, loss_pi = 1.0, 0.0, 0, loss_before
         for i in range(self.SEARCH_STEPS):
             pol.actor_flat().copy_(theta_old + step_frac * step)
             o = self._eval(data, advantage, None)
@@ -662,128 +683,25 @@ class TrustRegionUpdate:
             elif kl > kl_target:
                 self._log("INFO: violated KL constraint.")
             else:
-                acceptance, final_kl, accepted = i + 1, kl, True
+                acceptance, final_kl = i + 1, kl
                 self._log(f"Accept step at i={acceptance}")
                 break
             step_frac *= 0.8
-        if not accepted:
-            self._log("INFO: no suitable step found...")
-            step = torch.zeros_like(step)
-            acceptance = 0
-        pol.actor_flat().copy_(theta_old + step_frac * step)
-        return {"Misc/Alpha": alpha.item(), "Misc/FinalStepNorm": float(torch.norm(step)), "Misc/xHx": xHx.item(),
-                "Misc/gradient_norm": float(sc[2].sqrt()), "Misc/H_inv_g": float(sc[3].sqrt()), "Misc/AcceptanceStep": acceptance,
+        return {**self._finish(theta_old, step, step_frac, acceptance, sc, alpha),
                 "Loss/Loss_actor": loss_pi, "Train/KL": final_kl, "step_frac": step_frac}
-
 
     def run_npg(self, data, advantage):
         """natural_pg.py:355-387 / rcpo.py: the TRPO direction at full length, no line search."""
-        pol, kl_target = self.policy, self.cfg["target_kl"]
-        theta_old = pol.actor_flat().clone()
-        loss0 = self._grad(data, advantage, self.g)
-        self._old_dist(data)
-        self._cg(data, self.g, self.x)
-        self._fvp(data, self.x, self.Fx)
-        sc = torch.stack([torch.dot(self.x, self.Fx), loss0[0], torch.dot(self.g, self.g), torch.dot(self.x, self.x)]).cpu()
-        xHx = sc[0]
-        assert torch.isfinite(self.x).all(), "x is not finite"
-        assert xHx.item() >= 0, "xHx is negative"
-        alpha = torch.sqrt(2 * kl_target / (xHx + 1e-8))
+        theta_old, loss0 = self._direction(data, advantage)
+        sc, alpha = self._scalars(loss0)
         step = self.x * alpha.item()
-        pol.actor_flat().copy_(theta_old + step)
+        self.policy.actor_flat().copy_(theta_old + step)
         o = self._eval(data, advantage, None)           # KL(old || new).mean() at the new parameters
-        return {"Misc/Alpha": alpha.item(), "Misc/FinalStepNorm": float(torch.norm(step)), "Misc/xHx": xHx.item(),
-                "Misc/gradient_norm": float(sc[2].sqrt()), "Misc/H_inv_g": float(sc[3].sqrt()),
-                "Loss/Loss_actor": -float(sc[1]), "Train/KL": float(o[2])}
-
-
-def run_trust_region(args, config, algo, env=None, max_epochs=None, quiet=False, dp=None):
-    """main() of cpo.py / trpo_lag.py and their siblings trpo.py / natural_pg.py / rcpo.py.
-    ``dp``: a safepo.common.dist.DataParallel when launched one process per GPU (envs sharded; g, b, every FVP result and
-    the line-search means averaged over the ranks; the critics' gradients summed inside the update kernel)."""
-    seed_all(args.seed)
-    if args.device != "cuda":
-        raise L.SpoError("this build has no CPU path: run with --device cuda")
-    device = torch.device(f"cuda:{args.device_id}")
-    torch.cuda.set_device(device)
-    if env is None:
-        env, obs_space, act_space = make_env(args)
-    else:
-        obs_space, act_space = env.observation_space, env.action_space
-    T = args.steps_per_epoch // args.num_envs
-    epochs = args.total_steps // args.steps_per_epoch
-    policy = ActorVCritic(obs_space.shape[0], act_space.shape[0], config["hidden_sizes"]).to(device)
-    buffer = VectorizedOnPolicyBuffer(obs_space, act_space, size=T, device=device, num_envs=args.num_envs,
-                                      gamma=config["gamma"], gae_mode=getattr(args, "gae", "scan"))
-    lagrange = None
-    if algo in ("trpo_lag", "rcpo"):
-        lagrange = Lagrange(args.cost_limit, args.lagrangian_multiplier_init, args.lagrangian_multiplier_lr)
-    dict_args = dict(vars(args))
-    dict_args.update(config)
-    logger = EpochLogger(args.log_dir, seed=str(args.seed), verbose=not quiet, use_tensorboard=not quiet)
-    logger.save_config(dict_args)
-    logger.setup_torch_saver(policy.actor)
-    logger.log("Start with training.")
-    host_rng = getattr(args, "rng", "device") == "host"
-    roll_cls = DeviceTapeRollout if getattr(args, "resident_env", False) else Rollout
-    roll = roll_cls(env, policy, buffer, logger, args, device)
-    trust = TrustRegionUpdate(policy, config, device, logger=None if quiet else logger, dp=dp)
-    critics = CriticRegression(policy, config, host_rng, device, dp=dp)
-    red = None if dp is None else dp.all_reduce_sum
-
-    def jc():
-        return logger.get_stats("Metrics/EpCost") if dp is None else dp.mean_episode_cost(logger, device=device)
-    timings = []
-    n_epochs = epochs if max_epochs is None else min(epochs, max_epochs)
-    for epoch in range(n_epochs):
-        t_roll = roll.run(T)
-        t1 = time.time()
-        if algo in ("trpo_lag", "rcpo"):
-            lagrange.update_lagrange_multiplier(jc())
-            data = buffer.get(lagrange.lagrangian_multiplier, all_reduce=red)
-            res = trust.run_trpo(data, data["adv"]) if algo == "trpo_lag" else trust.run_npg(data, data["adv"])
-        elif algo in ("trpo", "natural_pg"):       # trpo.py:361: advantage = adv_r
-            data = buffer.get(0.0, all_reduce=red)
-            res = trust.run_trpo(data, data["adv"]) if algo == "trpo" else trust.run_npg(data, data["adv"])
-        else:
-            data = buffer.get(0.0, all_reduce=red)
-            ep_costs = jc() - args.cost_limit
-            res = trust.run_cpo(data, ep_costs, variant="pcpo" if algo == "pcpo" else "cpo")
-        cres = critics.run(data)
-        buffer.reset_segments()
-        torch.cuda.synchronize()
-        t_upd = time.time() - t1
-        timings.append({"rollout": t_roll, "update": t_upd, "steps": cres["steps"], "acceptance": res.get("Misc/AcceptanceStep")})
-        logger.store(**{k: v for k, v in res.items() if k.startswith(("Misc/", "Loss/", "Train/"))})
-        logger.store(**{"Loss/Loss_reward_critic": cres["loss_r"], "Loss/Loss_cost_critic": cres["loss_c"]})
-        if not logger.logged:
-            for k in ("Metrics/EpRet", "Metrics/EpCost", "Metrics/EpLen"):
-                logger.log_tabular(k)
-            logger.log_tabular("Train/Epoch", epoch + 1)
-            logger.log_tabular("Train/TotalSteps", (epoch + 1) * args.steps_per_epoch)
-            if lagrange is not None:
-                logger.log_tabular("Train/LagragianMultiplier", lagrange.lagrangian_multiplier)
-            logger.log_tabular("Train/KL")
-            for k in ("Loss/Loss_reward_critic", "Loss/Loss_cost_critic", "Loss/Loss_actor"):
-                logger.log_tabular(k)
-            logger.log_tabular("Time/Rollout", t_roll)
-            logger.log_tabular("Time/Update", t_upd)
-            logger.log_tabular("Time/Total", t_roll + t_upd)
-            logger.log_tabular("Value/RewardAdv", data["adv_r"].mean().item())
-            logger.log_tabular("Value/CostAdv", data["adv_c"].mean().item())
-            for k in ("Misc/Alpha", "Misc/FinalStepNorm", "Misc/xHx", "Misc/gradient_norm", "Misc/H_inv_g") + \
-                    (() if algo in ("natural_pg", "rcpo") else ("Misc/AcceptanceStep",)):
-                logger.log_tabular(k)
-            logger.dump_tabular()
-            if (epoch + 1) % 100 == 0 or epoch == 0:
-                logger.torch_save(itr=epoch)
-                logger.save_state({"Normalizer": _normalizer_state(roll, env)}, itr=epoch)
-    logger.close()
-    return policy, logger, timings, {"rollout": roll, "trust": trust, "critics": critics, "lagrange": lagrange, "buffer": buffer}
+        return {**self._misc(sc, alpha, step), "Loss/Loss_actor": -float(sc[1]), "Train/KL": float(o[2])}
 
 
 # ---------------------------------------------------------------------------------------
-# generic main() of the PPO-family scripts
+# main() of the two families
 # ---------------------------------------------------------------------------------------
 
 def make_env(args):
@@ -794,9 +712,9 @@ def make_env(args):
     return make_synthetic_env(args.num_envs, args.task, args.seed, episode_len=getattr(args, "episode_len", 1000))
 
 
-def run_policy_gradient(args, config, algo, env=None, max_epochs=None, quiet=False, dp=None):
-    """main() of ppo_lag.py / focops.py.  Returns (policy, logger, per-epoch timing list).
-    ``dp``: a safepo.common.dist.DataParallel when launched one process per GPU."""
+def _setup(args, config, env, quiet):
+    """Seeding, device, env, policy, buffer, logger and rollout loop of every main() (ppo_lag.py:69-147).
+    Returns (device, policy, buffer, logger, rollout); the rollout holds the env."""
     seed_all(args.seed)
     if args.device != "cuda":
         raise L.SpoError("this build has no CPU path: run with --device cuda")
@@ -806,81 +724,127 @@ def run_policy_gradient(args, config, algo, env=None, max_epochs=None, quiet=Fal
         env, obs_space, act_space = make_env(args)
     else:
         obs_space, act_space = env.observation_space, env.action_space
-    T = args.steps_per_epoch // args.num_envs
-    epochs = args.total_steps // args.steps_per_epoch
     policy = ActorVCritic(obs_space.shape[0], act_space.shape[0], config["hidden_sizes"]).to(device)
-    buffer = VectorizedOnPolicyBuffer(obs_space, act_space, size=T, device=device, num_envs=args.num_envs,
-                                      gamma=config["gamma"], gae_mode=getattr(args, "gae", "scan"))
-    # siblings of ppo_lag.py (SURVEY 8f rank 2): ppo.py / pg.py drop the multiplier, cppo_pid.py swaps in the PID one
-    CUP_LAMBDA, CUP_NU = 0.95, 0.20       # cup.py:45-46
-    if algo in ("ppo", "pg"):
-        lagrange = None
-    elif algo == "cppo_pid":
-        lagrange = PIDLagrangian(args.cost_limit, args.lagrangian_multiplier_init)
-    else:
-        lagrange = Lagrange(args.cost_limit, args.lagrangian_multiplier_init, args.lagrangian_multiplier_lr,
-                            lagrangian_upper_bound=2.0 if algo == "focops" else (CUP_NU if algo == "cup" else None))
-    dict_args = dict(vars(args))
-    dict_args.update(config)
+    buffer = VectorizedOnPolicyBuffer(obs_space, act_space, size=args.steps_per_epoch // args.num_envs, device=device,
+                                      num_envs=args.num_envs, gamma=config["gamma"], gae_mode=getattr(args, "gae", "scan"))
     logger = EpochLogger(args.log_dir, seed=str(args.seed), verbose=not quiet, use_tensorboard=not quiet)
-    logger.save_config(dict_args)
+    logger.save_config({**vars(args), **config})
     logger.setup_torch_saver(policy.actor)
     logger.log("Start with training.")
-    host_rng = getattr(args, "rng", "device") == "host"
     roll_cls = DeviceTapeRollout if getattr(args, "resident_env", False) else Rollout
-    roll = roll_cls(env, policy, buffer, logger, args, device)
-    kind = {"ppo_lag": L.LOSS_PPO_CLIP, "ppo": L.LOSS_PPO_CLIP, "cppo_pid": L.LOSS_PPO_CLIP, "cup": L.LOSS_PPO_CLIP, "pg": L.LOSS_PG,
-            "focops": L.LOSS_FOCOPS}[algo]
-    upd = PolicyGradientUpdate(policy, config, kind, epochs, host_rng, device, dp=dp)
+    return device, policy, buffer, logger, roll_cls(env, policy, buffer, logger, args, device)
+
+
+def _mean_episode_cost(logger, dp, device):
+    return logger.get_stats("Metrics/EpCost") if dp is None else dp.mean_episode_cost(logger, device=device)
+
+
+def _log_epoch(logger, roll, args, epoch, train, t_roll, t_upd, data, misc=()):
+    """One row of progress.csv once an episode has finished since the last row: the episode metrics, Train/Epoch,
+    Train/TotalSteps, the family's ``train`` columns (value None: the mean of the stored values), the losses, timings and
+    mean advantages, then the ``misc`` columns.  Checkpoints the actor and the observation statistics at the first epoch
+    and every 100th."""
+    if logger.logged:
+        return
+    for k in ("Metrics/EpRet", "Metrics/EpCost", "Metrics/EpLen"):
+        logger.log_tabular(k)
+    logger.log_tabular("Train/Epoch", epoch + 1)
+    logger.log_tabular("Train/TotalSteps", (epoch + 1) * args.steps_per_epoch)
+    for k, v in train.items():
+        logger.log_tabular(k, v)
+    for k in ("Loss/Loss_reward_critic", "Loss/Loss_cost_critic", "Loss/Loss_actor"):
+        logger.log_tabular(k)
+    logger.log_tabular("Time/Rollout", t_roll)
+    logger.log_tabular("Time/Update", t_upd)
+    logger.log_tabular("Time/Total", t_roll + t_upd)
+    logger.log_tabular("Value/RewardAdv", data["adv_r"].mean().item())
+    logger.log_tabular("Value/CostAdv", data["adv_c"].mean().item())
+    for k in misc:
+        logger.log_tabular(k)
+    logger.dump_tabular()
+    if (epoch + 1) % 100 == 0 or epoch == 0:
+        logger.torch_save(itr=epoch)
+        logger.save_state({"Normalizer": _normalizer_state(roll)}, itr=epoch)
+
+
+def _multiplier_columns(lagrange):
+    return {} if lagrange is None else {"Train/LagragianMultiplier": lagrange.lagrangian_multiplier}
+
+
+def run_trust_region(args, config, algo, env=None, max_epochs=None, quiet=False, dp=None):
+    """main() of cpo.py / trpo_lag.py and their siblings (TR_ALGOS).
+    ``dp``: a safepo.common.dist.DataParallel when launched one process per GPU (envs sharded; g, b, every FVP result and
+    the line-search means averaged over the ranks; the critics' gradients summed inside the update kernel)."""
+    method, multiplier, logs_acceptance = TR_ALGOS[algo]
+    device, policy, buffer, logger, roll = _setup(args, config, env, quiet)
+    lagrange = None if multiplier is None else multiplier(args)
+    trust = TrustRegionUpdate(policy, config, device, logger=None if quiet else logger, dp=dp)
+    critics = CriticRegression(policy, config, roll.host_rng, device, dp=dp)
+    red = None if dp is None else dp.all_reduce_sum
+    misc = ("Misc/Alpha", "Misc/FinalStepNorm", "Misc/xHx", "Misc/gradient_norm", "Misc/H_inv_g") + \
+        (("Misc/AcceptanceStep",) if logs_acceptance else ())
     timings = []
-    n_epochs = epochs if max_epochs is None else min(epochs, max_epochs)
-    for epoch in range(n_epochs):
-        t_roll = roll.run(T)
+    epochs = args.total_steps // args.steps_per_epoch
+    for epoch in range(epochs if max_epochs is None else min(epochs, max_epochs)):
+        t_roll = roll.run(buffer.size)
         t1 = time.time()
-        ep_costs = logger.get_stats("Metrics/EpCost") if dp is None else dp.mean_episode_cost(logger, device=device)
+        if lagrange is not None:
+            lagrange.update_lagrange_multiplier(_mean_episode_cost(logger, dp, device))
+        # without a multiplier the advantage is adv_r itself (trpo.py:361): (adv_r - 0 * adv_c) / 1, exactly
+        data = buffer.get(0.0 if lagrange is None else lagrange.lagrangian_multiplier, all_reduce=red)
+        if method == "trpo":
+            res = trust.run_trpo(data, data["adv"])
+        elif method == "npg":
+            res = trust.run_npg(data, data["adv"])
+        else:
+            res = trust.run_cpo(data, _mean_episode_cost(logger, dp, device) - args.cost_limit, variant=method)
+        cres = critics.run(data)
+        torch.cuda.synchronize()
+        t_upd = time.time() - t1
+        timings.append({"rollout": t_roll, "update": t_upd, "steps": cres["steps"], "acceptance": res.get("Misc/AcceptanceStep")})
+        logger.store(**{k: v for k, v in res.items() if k.startswith(("Misc/", "Loss/", "Train/"))})
+        logger.store(**{"Loss/Loss_reward_critic": cres["loss_r"], "Loss/Loss_cost_critic": cres["loss_c"]})
+        _log_epoch(logger, roll, args, epoch, {**_multiplier_columns(lagrange), "Train/KL": None}, t_roll, t_upd, data, misc)
+    logger.close()
+    return policy, logger, timings, {"rollout": roll, "trust": trust, "critics": critics, "lagrange": lagrange, "buffer": buffer}
+
+
+def run_policy_gradient(args, config, algo, env=None, max_epochs=None, quiet=False, dp=None):
+    """main() of ppo_lag.py / focops.py and their siblings (PG_ALGOS).  Returns (policy, logger, per-epoch timing list, parts).
+    ``dp``: a safepo.common.dist.DataParallel when launched one process per GPU."""
+    kind, multiplier = PG_ALGOS[algo]
+    device, policy, buffer, logger, roll = _setup(args, config, env, quiet)
+    lagrange = None if multiplier is None else multiplier(args)
+    epochs = args.total_steps // args.steps_per_epoch
+    upd = PolicyGradientUpdate(policy, config, kind, epochs, roll.host_rng, device, dp=dp)
+    red = None if dp is None else dp.all_reduce_sum
+    timings = []
+    for epoch in range(epochs if max_epochs is None else min(epochs, max_epochs)):
+        t_roll = roll.run(buffer.size)
+        t1 = time.time()
+        ep_costs = _mean_episode_cost(logger, dp, device)
         if lagrange is not None:
             lagrange.update_lagrange_multiplier(ep_costs)
         # without a multiplier the advantage is adv_r itself (ppo.py:272): (adv_r - 0 * adv_c) / 1, exactly
         lam = lagrange.lagrangian_multiplier if lagrange is not None else 0.0
-        # cup.py:284: the first stage is plain PPO on adv_r; the multiplier enters the projection stage only
-        data = buffer.get(0.0 if algo == "cup" else lam, all_reduce=None if dp is None else dp.all_reduce_sum)
         if algo == "cup":
+            # cup.py:284: the first stage is plain PPO on adv_r; the multiplier enters the projection stage only
+            data = buffer.get(0.0, all_reduce=red)
             res = upd.run(data, step_sched=False)
             coef = (1 - config["gamma"] * CUP_LAMBDA) / (1 - config["gamma"])
-            data2 = dict(data)
-            data2["adv"] = data["adv_c"].reshape(-1)
-            res2 = upd.run(data2, kind=L.LOSS_CUP_PROJECTION, cup_coef=lam * coef)
-            res["second_stop_iter"], res["kl"], res["steps"] = res2["stop_iter"], res2["kl"], res["steps"] + res2["steps"]
+            res2 = upd.run({**data, "adv": data["adv_c"].reshape(-1)}, kind=L.LOSS_CUP_PROJECTION, cup_coef=lam * coef)
+            stop_iters = {"Train/StopIter": res["stop_iter"], "Train/SeconStageStopIter": res2["stop_iter"]}
+            res["kl"], res["steps"] = res2["kl"], res["steps"] + res2["steps"]
         else:
+            data = buffer.get(lam, all_reduce=red)
             res = upd.run(data)
-        buffer.reset_segments()
+            stop_iters = {"Train/StopIter": res["stop_iter"]}
         torch.cuda.synchronize()
         t_upd = time.time() - t1
         timings.append({"rollout": t_roll, "update": t_upd, "stop_iter": res["stop_iter"], "steps": res["steps"]})
         logger.store(**{"Loss/Loss_reward_critic": res["loss_r"], "Loss/Loss_cost_critic": res["loss_c"],
                         "Loss/Loss_actor": res["loss_pi"]})
-        if not logger.logged:
-            for k in ("Metrics/EpRet", "Metrics/EpCost", "Metrics/EpLen"):
-                logger.log_tabular(k)
-            logger.log_tabular("Train/Epoch", epoch + 1)
-            logger.log_tabular("Train/TotalSteps", (epoch + 1) * args.steps_per_epoch)
-            logger.log_tabular("Train/StopIter", res["stop_iter"])
-            if algo == "cup":
-                logger.log_tabular("Train/SeconStageStopIter", res["second_stop_iter"])
-            logger.log_tabular("Train/KL", res["kl"])
-            if lagrange is not None:
-                logger.log_tabular("Train/LagragianMultiplier", lagrange.lagrangian_multiplier)
-            logger.log_tabular("Train/LR", upd.sched.lr)
-            for k in ("Loss/Loss_reward_critic", "Loss/Loss_cost_critic", "Loss/Loss_actor"):
-                logger.log_tabular(k)
-            logger.log_tabular("Time/Rollout", t_roll)
-            logger.log_tabular("Time/Update", t_upd)
-            logger.log_tabular("Time/Total", t_roll + t_upd)
-            logger.log_tabular("Value/RewardAdv", data["adv_r"].mean().item())
-            logger.log_tabular("Value/CostAdv", data["adv_c"].mean().item())
-            logger.dump_tabular()
-            if (epoch + 1) % 100 == 0 or epoch == 0:
-                logger.torch_save(itr=epoch)
-                logger.save_state({"Normalizer": _normalizer_state(roll, env)}, itr=epoch)
+        train = {**stop_iters, "Train/KL": res["kl"], **_multiplier_columns(lagrange), "Train/LR": upd.sched.lr}
+        _log_epoch(logger, roll, args, epoch, train, t_roll, t_upd, data)
     logger.close()
     return policy, logger, timings, {"rollout": roll, "update": upd, "lagrange": lagrange, "buffer": buffer}
