@@ -350,6 +350,41 @@ int spo_ma_lagrange_step(const float* imp, const float* cost_adv, const float* a
 int spo_ma_clip_adam(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int count, float max_grad_norm, double lr, double beta1,
                      double beta2, double eps, double weight_decay, int step, float* work, float* norm_out, void* stream);
 
+/* ---- MACPO trust region on the multi-agent nets (safepo/multi_agent/macpo.py:153-380; csrc/spo_ma_trust.cu) ----
+ * The Fisher-vector product of fisher_vector_product (macpo.py:187-198: double backprop of kl_divergence, :153-166) in closed form:
+ * spo_ma_ln_in_jvp: tangent of the input LayerNorm, out[n][K] = dln_w xhat + dln_b (the observations carry no tangent).
+ * spo_ma_gemm_nt_pair: C[M][N] = A1[M][K1] B1[N][K1]^T + A2[M][K2] B2[N][K2]^T (+ bias[N], may be NULL): the tangent
+ *   z' = x' W^T + x W'^T + b' of a Linear layer (and mu' of the mean head).
+ * spo_ma_ln_elu_jvp: in place on t[n][H]: z' -> y' through ELU (kept pre = ELU(z)) and LayerNorm (ln_w; tangents dln_w, dln_b).
+ * spo_ma_fvp_head: dmean[n][A] = dmu * 2 / (1e-8 + 2 std^2) / n, part[ceil(n/32)][A] = per-CTA column sums (the mean bias).
+ * spo_ma_fvp_finish: out = g + damping v on a packed buffer, except out[ls_off + j] = (h_j + damping) v[ls_off + j] with h the
+ *   log_std block of the reference's KL, whose log term has the sign of KL(new || old)'s (macpo.py:163-164):
+ *   h = f_ss s'^2 + f_s s'', f_s = -1/s - 4 s^3 / D^2, f_ss = 1/s^2 - 4 s^2 / D^2 + 32 s^4 / D^3, D = 1e-8 + 2 s^2.
+ * Conjugate gradient (macpo.py:168-185) over `count` floats; state[4] = {rdotr, done, p.Ap, new rdotr}, part[256] scratch:
+ *   spo_ma_cg_begin: x = 0, r = p = b, rdotr = b.b.  spo_ma_cg_update: alpha = rdotr / (p.Ap + 1e-8), x += alpha p,
+ *   r -= alpha Ap, p = r + (r.r / rdotr) p; sets done once r.r < residual_tol, after which further updates are no-ops.
+ * spo_ma_dot: out = x.y (fixed-order two-stage sum).  spo_ma_axpby: out = a x + b y (y may be NULL).
+ * spo_ma_clip_norm: x *= max_norm / |x| when |x| > max_norm (macpo.py:343-345); nrm2 = x.x before.
+ * spo_ma_linesearch_eval (macpo.py:349-368): on the features of the trial weights, scalars[5] = {-mean(imp factor adv),
+ *   mean(imp factor cost_adv), mean_rows(sum_j kl_divergence), mean(imp), entropy}, imp = prod_j exp(logp_j - old_logp_j),
+ *   old_mean[n][A] / old_std[A] of the weights before the step.  part[ceil(n/32)][4] scratch. */
+int spo_ma_ln_in_jvp(const float* x, int n, int K, const float* dln_w, const float* dln_b, float* out, void* stream);
+int spo_ma_gemm_nt_pair(const float* A1, const float* B1, int K1, const float* A2, const float* B2, int K2, const float* bias, float* C, int M, int N,
+                    void* stream);
+int spo_ma_ln_elu_jvp(float* t, const float* pre, const float* ln_w, const float* dln_w, const float* dln_b, int n, int H, void* stream);
+int spo_ma_fvp_head(const float* dmu, int n, int A, const float* log_std, float std_x_coef, float std_y_coef, float* dmean, float* part,
+                    void* stream);
+int spo_ma_fvp_finish(const float* g, const float* v, int count, int ls_off, int A, const float* log_std, float std_x_coef, float std_y_coef,
+                      float damping, float* out, void* stream);
+int spo_ma_dot(const float* x, const float* y, int count, float* part, float* out, void* stream);
+int spo_ma_cg_begin(const float* b, float* x, float* r, float* p, int count, float* state, float* part, void* stream);
+int spo_ma_cg_update(float* p, const float* Ap, float* x, float* r, int count, float* state, float* part, float residual_tol, void* stream);
+int spo_ma_axpby(float* out, float a, const float* x, float b, const float* y, int count, void* stream);
+int spo_ma_clip_norm(float* x, int count, float max_norm, float* part, float* nrm2, void* stream);
+int spo_ma_linesearch_eval(const float* feat, int n, int H, const float* W, const float* b, const float* log_std, int A, const float* actions,
+                           const float* old_logp, const float* adv, const float* cost_adv, const float* factor, const float* old_mean,
+                           const float* old_std, float std_x_coef, float std_y_coef, float* part, float* scalars, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -112,6 +112,17 @@ _ABI = {
     "spo_ma_popart_normalize": ([_p, _i, _p, _d, _f, _p, _p], True),
     "spo_ma_lagrange_step": ([_p, _p, _p, _i, _f, _d, _f, _p, _p], True),
     "spo_ma_clip_adam": ([_p, _p, _p, _p, _i, _f, _d, _d, _d, _d, _d, _i, _p, _p, _p], True),
+    "spo_ma_ln_in_jvp": ([_p, _i, _i, _p, _p, _p, _p], True),
+    "spo_ma_gemm_nt_pair": ([_p, _p, _i, _p, _p, _i, _p, _p, _i, _i, _p], True),
+    "spo_ma_ln_elu_jvp": ([_p, _p, _p, _p, _p, _i, _i, _p], True),
+    "spo_ma_fvp_head": ([_p, _i, _i, _p, _f, _f, _p, _p, _p], True),
+    "spo_ma_fvp_finish": ([_p, _p, _i, _i, _i, _p, _f, _f, _f, _p, _p], True),
+    "spo_ma_dot": ([_p, _p, _i, _p, _p, _p], True),
+    "spo_ma_cg_begin": ([_p, _p, _p, _p, _i, _p, _p, _p], True),
+    "spo_ma_cg_update": ([_p, _p, _p, _p, _i, _p, _p, _f, _p], True),
+    "spo_ma_axpby": ([_p, _f, _p, _f, _p, _i, _p], True),
+    "spo_ma_clip_norm": ([_p, _i, _f, _p, _p, _p], True),
+    "spo_ma_linesearch_eval": ([_p, _i, _i, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _f, _f, _p, _p, _p], True),
 }
 EXPORTS = tuple(_ABI)
 _KERNEL_CALLS = frozenset(name for name, (_, launch) in _ABI.items() if launch)

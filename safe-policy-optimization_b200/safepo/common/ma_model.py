@@ -306,3 +306,230 @@ class MultiAgentTrainer:
             out = self.ppo_update(buf.whole_batch_sample(advantages, cost_adv, perm))
         return out
 
+
+def macpo_case(q_coef, r_coef, s_coef, bb, rescale_constraint_val, target_kl):
+    """The optim_case analysis of MACPO_Trainer.trpo_update (macpo.py:271-321) on host float32 tensors, with every 1e-8
+    substitution of the reference: returns (optim_case, lam, nu, whether_recover_policy_value) as Python floats / int."""
+    inf = float("inf")
+    if bb <= 1e-8 and rescale_constraint_val < 0:
+        optim_case, whether = 4, torch.tensor(0.0)
+    else:
+        if r_coef == 0:
+            r_coef = torch.tensor(1e-8)
+        if s_coef == 0:
+            s_coef = torch.tensor(1e-8)
+        positive_cauchy = q_coef - r_coef ** 2 / (1e-8 + s_coef)
+        whether = 2 * target_kl - rescale_constraint_val ** 2 / (1e-8 + s_coef)
+        if rescale_constraint_val < 0:
+            optim_case = 3 if whether < 0 else 2
+        else:
+            optim_case = 1 if whether >= 0 else 0
+    if whether == 0:
+        whether = torch.tensor(1e-8)
+    if optim_case in (3, 4):
+        lam, nu = torch.sqrt(q_coef / (2 * target_kl)), torch.tensor(0.0)
+    elif optim_case in (1, 2):
+        LA, LB = [0.0, r_coef / rescale_constraint_val], [r_coef / rescale_constraint_val, inf]
+        LA, LB = (LA, LB) if rescale_constraint_val < 0 else (LB, LA)
+        proj = lambda x, L: max(L[0], min(L[1], x))      # noqa: E731
+        lam_a = proj(torch.sqrt(positive_cauchy / whether), LA)
+        lam_b = proj(torch.sqrt(q_coef / torch.tensor(2 * target_kl)), LB)
+        f_a = -0.5 * (positive_cauchy / (1e-8 + lam_a) + whether * lam_a) - r_coef * rescale_constraint_val / (1e-8 + s_coef)
+        f_b = -0.5 * (q_coef / (1e-8 + lam_b) + 2 * target_kl * lam_b)
+        lam = lam_a if f_a >= f_b else lam_b
+        nu = max(0, lam * rescale_constraint_val - r_coef) / (1e-8 + s_coef)
+    else:
+        lam, nu = torch.tensor(0.0), torch.sqrt(torch.tensor(2 * target_kl) / (1e-8 + s_coef))
+    return optim_case, float(lam), float(nu), float(whether)
+
+
+class MACPOTrainer(MultiAgentTrainer):
+    """``MACPO_Trainer`` for one agent (macpo.py:96-414): both critics as in MAPPO-Lag, the actor moved by a constrained
+    trust-region step.  Per update: the surrogate gradients g (reward) and b (cost) through the actor backward chain, two conjugate-
+    gradient solves of ``conjugate_gradient_iters`` Fisher-vector products each (forward tangents + the backward chain, the
+    reference's quirky log_std block, damping 0.1), ONE device -> host read of the stacked scalars for the case analysis, then a
+    backtracking line search with one read per trial.  ``cfg`` adds target_kl, searching_steps, conjugate_gradient_iters,
+    step_fraction and fraction_coef to the MAPPO-Lag keys (actor_lr, entropy_coef, lagrangian_coef_rate, lamda_lagr unused)."""
+
+    DAMPING, RESIDUAL_TOL, MAX_STEP_NORM = 0.1, 1e-10, 0.5        # macpo.py:198, :169, :344
+
+    def __init__(self, nets: MultiAgentNets, cfg):
+        super().__init__(nets, dict({"lamda_lagr": 0.0}, **dict(cfg)))
+        self._tr = {}
+        net, dev = nets.actor, self.device
+        base = net.flat.data_ptr()
+        self._off = {k: (v.data_ptr() - base) // 4 for k, v in net.p.items()}
+        self._count = net.flat.numel()
+        f = dict(dtype=torch.float32, device=dev)
+        self._vec = {k: torch.zeros(self._count, **f) for k in ("g", "b", "gsd", "bsd", "x", "r", "p", "Ap", "old")}
+        self._cg_state = torch.zeros(4, **f)
+        self._dpart = torch.empty(256, **f)
+        self._lam = torch.tensor([0.0, 1.0], **f)
+
+    def _tangents(self, v):
+        """Views of a packed vector under the actor's parameter names."""
+        return {k: v[o:o + p.numel()].view(p.shape) for (k, p), o in zip(self.nets.actor.p.items(), self._off.values())}
+
+    def _trust_ws(self, n, net):
+        key = (n, net.D, net.H)
+        if key not in self._tr:
+            f = dict(dtype=torch.float32, device=self.device)
+            A = self.nets.act_dim
+            self._tr[key] = dict(ta=torch.empty(n, net.H, **f), tb=torch.empty(n, net.H, **f), txn=torch.empty(n, net.D, **f),
+                                 dmu=torch.empty(n, A, **f), old_mean=torch.empty(n, A, **f), zeros=torch.zeros(n, **f),
+                                 imp=torch.empty(n, 1, **f))
+        return self._tr[key]
+
+    def _surrogate_grad(self, net, feat, ws, obs, actions, old_logp, adv, cost_adv, factor, lamda, imp, scal, out):
+        """d/d actor of -mean(imp factor adv) (lamda -> 0) or of mean(imp factor cost_adv) (adv = 0, lamda -> 1), macpo.py:242-251:
+        the clipped-surrogate head with an unbounded clip range and no entropy term, then the actor's backward chain."""
+        n, A, nets = obs.shape[0], self.nets.act_dim, self.nets
+        wm, bm, ls = net.p["act.action_out.fc_mean.weight"], net.p["act.action_out.fc_mean.bias"], net.p["act.action_out.log_std"]
+        L.call("spo_ma_actor_loss", L.ptr(feat), n, net.H, L.ptr(wm), L.ptr(bm), L.ptr(ls), A, L.ptr(actions), L.ptr(old_logp), L.ptr(adv),
+               L.ptr(cost_adv), L.ptr(factor), L.ptr(lamda), float("-inf"), float("inf"), nets.std_x_coef, nets.std_y_coef, L.ptr(ws["dmean"]),
+               L.ptr(imp), L.ptr(ws["part"]), L.stream())
+        L.call("spo_ma_actor_finalize", L.ptr(ws["part"]), (n + 31) // 32, n, L.ptr(ls), A, nets.std_x_coef, nets.std_y_coef, 0.0,
+               L.ptr(net.g["act.action_out.fc_mean.bias"]), L.ptr(net.g["act.action_out.log_std"]), L.ptr(scal), L.stream())
+        self._gemm_tn(ws["dmean"], feat, net.g["act.action_out.fc_mean.weight"], n, A, net.H, ws)
+        L.call("spo_ma_gemm_nn", L.ptr(ws["dmean"]), L.ptr(wm), L.ptr(ws["dy"]), n, net.H, A, L.stream())
+        self._backward(net, obs, ws, ws["dy"])
+        out.copy_(net.gflat)
+
+    def fvp(self, obs, v, out, ws=None, tw=None):
+        """out = F v + 0.1 v at the actor's current weights on the rows ``obs`` (macpo.py:187-198).  The training forward's
+        activations (ws['xn'], ws['pre'], ws['out']) must be those of ``obs``: pass the workspace of a _forward_train on it, or
+        leave ws None to run one."""
+        net, nets = self.nets.actor, self.nets
+        n, H, A = obs.shape[0], net.H, nets.act_dim
+        if ws is None:
+            ws = self._ws(n, net)
+            self._forward_train(net, obs, ws)
+        tw = tw or self._trust_ws(n, net)
+        p, t = net.p, self._tangents(v)
+        L.call("spo_ma_ln_in_jvp", L.ptr(obs), n, net.D, L.ptr(t["base.feature_norm.weight"]), L.ptr(t["base.feature_norm.bias"]),
+               L.ptr(tw["txn"]), L.stream())
+        x, dx, dst = ws["xn"], tw["txn"], tw["ta"]
+        for i, (w, bb, lw, lb) in enumerate(net.blocks):
+            K = net.D if i == 0 else H
+            L.call("spo_ma_gemm_nt_pair", L.ptr(dx), L.ptr(p[w]), K, L.ptr(x), L.ptr(t[w]), K, L.ptr(t[bb]), L.ptr(dst), n, H, L.stream())
+            L.call("spo_ma_ln_elu_jvp", L.ptr(dst), L.ptr(ws["pre"][i]), L.ptr(p[lw]), L.ptr(t[lw]), L.ptr(t[lb]), n, H, L.stream())
+            x, dx, dst = ws["out"][i], dst, (tw["tb"] if dst is tw["ta"] else tw["ta"])
+        wm, ls = p["act.action_out.fc_mean.weight"], p["act.action_out.log_std"]
+        L.call("spo_ma_gemm_nt_pair", L.ptr(dx), L.ptr(wm), H, L.ptr(x), L.ptr(t["act.action_out.fc_mean.weight"]), H,
+               L.ptr(t["act.action_out.fc_mean.bias"]), L.ptr(tw["dmu"]), n, A, L.stream())
+        L.call("spo_ma_fvp_head", L.ptr(tw["dmu"]), n, A, L.ptr(ls), nets.std_x_coef, nets.std_y_coef, L.ptr(ws["dmean"]), L.ptr(ws["part"]),
+               L.stream())
+        L.call("spo_ma_partial_reduce", L.ptr(ws["part"]), (n + 31) // 32, A, 1, A, L.ptr(net.g["act.action_out.fc_mean.bias"]), None, None,
+               1.0, L.stream())
+        self._gemm_tn(ws["dmean"], x, net.g["act.action_out.fc_mean.weight"], n, A, H, ws)
+        L.call("spo_ma_gemm_nn", L.ptr(ws["dmean"]), L.ptr(wm), L.ptr(ws["dy"]), n, H, A, L.stream())
+        self._backward(net, obs, ws, ws["dy"])
+        L.call("spo_ma_fvp_finish", L.ptr(net.gflat), L.ptr(v), self._count, self._off["act.action_out.log_std"], A, L.ptr(ls),
+               nets.std_x_coef, nets.std_y_coef, self.DAMPING, L.ptr(out), L.stream())
+        return out
+
+    def _cg(self, obs, ws, tw, rhs, sol):
+        """conjugate_gradient (macpo.py:168-185): conjugate_gradient_iters FVPs, no host synchronisation (the device stops
+        updating once the residual is below 1e-10)."""
+        V, st, c = self._vec, self._cg_state, self._count
+        L.call("spo_ma_cg_begin", L.ptr(rhs), L.ptr(sol), L.ptr(V["r"]), L.ptr(V["p"]), c, L.ptr(st), L.ptr(self._dpart), L.stream())
+        for _ in range(int(self.cfg["conjugate_gradient_iters"])):
+            self.fvp(obs, V["p"], V["Ap"], ws, tw)
+            L.call("spo_ma_cg_update", L.ptr(V["p"]), L.ptr(V["Ap"]), L.ptr(sol), L.ptr(V["r"]), c, L.ptr(st), L.ptr(self._dpart),
+                   self.RESIDUAL_TOL, L.stream())
+
+    def _dot(self, x, y, out):
+        L.call("spo_ma_dot", L.ptr(x), L.ptr(y), self._count, L.ptr(self._dpart), L.ptr(out), L.stream())
+
+    def trpo_update(self, sample):
+        """One MACPO update on the whole sample (a dict with the oracle's keys, or the reference's 18-tuple), macpo.py:200-380.
+        Returns a dict: value_loss, critic_grad_norm, cost_grad_norm (device), and as host floats kl, loss_improve,
+        expected_improve, dist_entropy, ratio (mean importance weight), cost_loss (the cost surrogate, as the reference returns it),
+        whether_recover_policy_value, lam, nu, optim_case, accepted (index of the accepted trial, -1 = all rejected, actor
+        restored); g, b, g_step_dir, b_step_dir, x are device copies of the flat vectors."""
+        if not isinstance(sample, dict):
+            sample = {k: v for k, v in zip(_SAMPLE_KEYS, sample)}
+        dev, c, nets = self.device, self.cfg, self.nets
+
+        def dv_(x, cols=None):
+            t = torch.as_tensor(x, dtype=torch.float32).to(dev).contiguous()
+            return t.reshape(t.shape[0], -1) if cols is None else t.reshape(-1)
+        obs, share_obs, actions, old_logp = dv_(sample["obs"]), dv_(sample["share_obs"]), dv_(sample["actions"]), dv_(sample["old_action_log_probs"])
+        value_preds, returns, adv, factor = dv_(sample["value_preds"], 1), dv_(sample["returns"], 1), dv_(sample["adv_targ"], 1), dv_(sample["factor"], 1)
+        cost_preds, cost_returns, cost_adv = dv_(sample["cost_preds"], 1), dv_(sample["cost_returns"], 1), dv_(sample["cost_adv_targ"], 1)
+        aver_costs = torch.as_tensor(sample["aver_episode_costs"], dtype=torch.float32).to(dev)
+        n, A = obs.shape[0], nets.act_dim
+
+        # ---- critics (macpo.py:220-231): the same update as MAPPO-Lag's, reward critic first ----
+        value_loss, critic_grad_norm = self._critic_update(nets.critic, share_obs, value_preds, returns, self._ws(n, nets.critic))
+        _, cost_grad_norm = self._critic_update(nets.cost_critic, share_obs, cost_preds, cost_returns, self._ws(n, nets.cost_critic))
+
+        # ---- surrogate gradients at the current actor (macpo.py:239-253); its activations stay valid until the line search ----
+        net, V = nets.actor, self._vec
+        ws, tw = self._ws(n, net), self._trust_ws(n, net)
+        feat = self._forward_train(net, obs, ws)
+        scal_r = torch.empty(2, dtype=torch.float32, device=dev)
+        scal_c = torch.empty(2, dtype=torch.float32, device=dev)
+        self._surrogate_grad(net, feat, ws, obs, actions, old_logp, adv, tw["zeros"], factor, self._lam[0:1], tw["imp"], scal_r, V["g"])
+        self._surrogate_grad(net, feat, ws, obs, actions, old_logp, tw["zeros"], cost_adv, factor, self._lam[1:2], tw["imp"], scal_c, V["b"])
+        wm, bm, ls = net.p["act.action_out.fc_mean.weight"], net.p["act.action_out.fc_mean.bias"], net.p["act.action_out.log_std"]
+        L.call("spo_ma_head", L.ptr(feat), n, net.H, L.ptr(wm), L.ptr(bm), A, L.ptr(ls), nets.std_x_coef, nets.std_y_coef, None,
+               L.ptr(tw["old_mean"]), None, L.stream())
+        old_std = (torch.sigmoid(ls / nets.std_x_coef) * nets.std_y_coef).contiguous()
+
+        # ---- the two natural directions (macpo.py:255-262) and the coefficients, read back once ----
+        self._cg(obs, ws, tw, V["g"], V["gsd"])
+        self._cg(obs, ws, tw, V["b"], V["bsd"])
+        dots = torch.empty(4, dtype=torch.float32, device=dev)
+        for i, (x_, y_) in enumerate(((V["g"], V["gsd"]), (V["g"], V["bsd"]), (V["b"], V["bsd"]), (V["b"], V["b"]))):
+            self._dot(x_, y_, dots[i:i + 1])
+        host = torch.cat([dots, scal_r[0:1], scal_c[0:1], aver_costs.mean().reshape(1)]).cpu()
+        q, r, s, bb, reward_loss, cost_loss = (host[i] for i in range(6))
+        rescale = (host[6] - c["cost_limit"]) * (1 - c["gamma"])
+        if rescale == 0:
+            rescale = torch.tensor(1e-8)
+        optim_case, lam, nu, whether = macpo_case(q, r, s, bb, rescale, float(c["target_kl"]))
+
+        # ---- the step x (macpo.py:323-325) and the line search (:337-378) ----
+        c1 = 1.0 / (lam + 1e-8) if optim_case > 0 else 0.0
+        c2 = (c1 * nu if optim_case > 0 else nu) if optim_case != 4 else 0.0
+        L.call("spo_ma_axpby", L.ptr(V["x"]), c1, L.ptr(V["gsd"]), c2, L.ptr(V["bsd"]), self._count, L.stream())
+        ls_dev = torch.empty(6, dtype=torch.float32, device=dev)
+        self._dot(V["x"], V["g"], ls_dev[5:6])
+        L.call("spo_ma_clip_norm", L.ptr(V["x"]), self._count, self.MAX_STEP_NORM, L.ptr(self._dpart), L.ptr(self._cg_state[2:3]), L.stream())
+        V["old"].copy_(net.flat)
+        fraction, coef = float(c["step_fraction"]), float(c["fraction_coef"])
+        limit = max(-float(rescale), 0.0)
+        accepted, expected_improve, row = -1, None, None
+        fbuf = nets._buffers(n, net.H)
+        for i in range(int(c["searching_steps"])):
+            L.call("spo_ma_axpby", L.ptr(net.flat), 1.0, L.ptr(V["old"]), -coef * fraction ** i, L.ptr(V["x"]), self._count, L.stream())
+            tfeat = net.features(obs, fbuf)
+            L.call("spo_ma_linesearch_eval", L.ptr(tfeat), n, net.H, L.ptr(wm), L.ptr(bm), L.ptr(ls), A, L.ptr(actions), L.ptr(old_logp), L.ptr(adv),
+                   L.ptr(cost_adv), L.ptr(factor), L.ptr(tw["old_mean"]), L.ptr(old_std), nets.std_x_coef, nets.std_y_coef, L.ptr(ws["part"]),
+                   L.ptr(ls_dev), L.stream())
+            row = ls_dev.cpu()
+            if expected_improve is None:
+                expected_improve = -float(row[5])
+            loss_improve = row[0] - reward_loss
+            if row[2] < c["target_kl"] and (loss_improve < 0 if optim_case > 1 else True) and float(row[1] - cost_loss) <= limit:
+                accepted = i
+                break
+            expected_improve *= fraction
+        if accepted < 0:
+            net.flat.copy_(V["old"])
+        return dict(value_loss=value_loss, critic_grad_norm=critic_grad_norm, cost_grad_norm=cost_grad_norm, kl=float(row[2]),
+                    loss_improve=float(loss_improve), expected_improve=float(expected_improve), dist_entropy=float(row[4]), ratio=float(row[3]),
+                    cost_loss=float(cost_loss), whether_recover_policy_value=whether, lam=lam, nu=nu, optim_case=optim_case, accepted=accepted,
+                    g=V["g"].clone(), b=V["b"].clone(), g_step_dir=V["gsd"].clone(), b_step_dir=V["bsd"].clone(), x=V["x"].clone())
+
+    def train(self, buf, perms=None):
+        """MACPO_Trainer.train (macpo.py:382-400): advantages = returns - denormalised predictions standardised with +1e-5 and no
+        masking, then ONE trpo_update on the whole batch.  ``perms``: the row order (a tensor, or a one-element list of one)."""
+        mean, sd = self.popart_mean_sqrt_var()
+
+        def standardise(ret, pred):
+            adv = ret[:-1] - (pred[:-1] * sd + mean)
+            return (adv - torch.mean(adv)) / (torch.std(adv) + 1e-5)
+        perm = perms[0] if isinstance(perms, (list, tuple)) else perms
+        return self.trpo_update(buf.whole_batch_sample(standardise(buf.returns, buf.value_preds), standardise(buf.cost_returns, buf.cost_preds), perm))

@@ -18,12 +18,14 @@ from safepo.common.ma_model import MultiAgentNets, MultiAgentTrainer
 
 
 class Runner:
+    trainer_cls = MultiAgentTrainer          # the per-agent trainer (macpo.Runner swaps in MACPOTrainer)
+
     def __init__(self, nets, config, obs_dim, share_obs_dim, act_dim):
         """``nets``: one MultiAgentNets per agent (all on the same device)."""
         self.config, self.num_agents = dict(config), len(nets)
         self.nets = list(nets)
         self.device = nets[0].device
-        self.trainer = [MultiAgentTrainer(n, self.config) for n in self.nets]
+        self.trainer = [self.trainer_cls(n, self.config) for n in self.nets]
         self.buffer = [SeparatedReplayBuffer(self.config, obs_dim, share_obs_dim, act_dim, self.device) for _ in self.nets]
         self.T, self.N = int(config["episode_length"]), int(config["n_rollout_threads"])
 
@@ -94,6 +96,13 @@ class Runner:
             b.after_update()
         return outs if collect_outputs else order
 
+    def _agent_log(self, a, out):
+        """The logged values of agent a's last update (mappolag.py:362-373)."""
+        value_loss, critic_norm, policy_loss, entropy, actor_norm, imp, cost_loss, cost_norm = out
+        return {f"Loss/Loss_reward_critic/agent{a}": float(value_loss), f"Loss/Loss_cost_critic/agent{a}": float(cost_loss),
+                f"Loss/Loss_actor/agent{a}": float(policy_loss), f"Misc/Entropy/agent{a}": float(entropy),
+                f"Misc/Ratio/agent{a}": float(imp.mean()), f"Misc/Lagrange/agent{a}": float(self.trainer[a].lamda_lagr)}
+
     def return_aver_cost(self, aver_episode_costs):
         for b in self.buffer:
             b.return_aver_insert(aver_episode_costs)
@@ -131,10 +140,7 @@ class Runner:
                 row["Metrics/EpCost"] = float(finished_cost.mean())
                 self.return_aver_cost(finished_cost.mean())          # mappolag.py:349-351
             for a, out in outs.items():                              # the reference logs the last update of every agent's train()
-                value_loss, critic_norm, policy_loss, entropy, actor_norm, imp, cost_loss, cost_norm = out
-                row.update({f"Loss/Loss_reward_critic/agent{a}": float(value_loss), f"Loss/Loss_cost_critic/agent{a}": float(cost_loss),
-                            f"Loss/Loss_actor/agent{a}": float(policy_loss), f"Misc/Entropy/agent{a}": float(entropy),
-                            f"Misc/Ratio/agent{a}": float(imp.mean()), f"Misc/Lagrange/agent{a}": float(self.trainer[a].lamda_lagr)})
+                row.update(self._agent_log(a, out))
             row["Time/Total"] = time.time() - start
             row["Time/FPS"] = int(row["Train/TotalSteps"] / max(row["Time/Total"], 1e-9))
             rows.append(row)
